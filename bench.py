@@ -3,7 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload c5|c1..c4] [--kind auto|merge|vector|light]
-                    [--exchange p2p|nccl] [--override SIZE]
+                    [--exchange p2p|nccl] [--override SIZE] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[4], the configuration the 1/2/4/8-GPU metric is quoted on):
 R-MAT scale 27, edge factor 16 (134M rows, 2^31 nonzeros, int64 offsets, fp32), row-sharded
@@ -25,6 +25,12 @@ One JSON line on stdout (rank 0):
 
 `--impl reference` times that CPU path alone (rank 0 only) and prints the same line with
 "impl": "reference".
+
+`--dump-outputs DIR` (own arm) writes, after the timed steps, what a caller of the power
+iteration receives from the last of them: DIR/x.npy (the iterate A x, not yet divided by its
+norm; a fixed seeded sample when it is larger than 32 MB) and DIR/eigen_estimate.npy (||A x||).
+The matrix and x0 are fixed by the seed, so two builds run with the same arguments can be
+compared output for output.
 """
 from __future__ import annotations
 
@@ -69,7 +75,15 @@ def parse_args():
     p.add_argument("--opts", default="", help="library options name=value,... (experiments; recorded in config)")
     p.add_argument("--no-configs", action="store_true",
                    help="skip the c1..c4 + cuSPARSE leg (N = 1 only; outside the timed region)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write the iterate x and the eigenvalue estimate as "
+                        "DIR/<name>.npy (own arm, rank 0)")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        p.error("--dump-outputs writes the own arm's outputs; the reference arm has none")
+    return args
 
 
 def measured_peak():
@@ -328,8 +342,11 @@ def reference_arm(args, rank, world):
             "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic"}
     have_gpu = False
     try:
+        # asked of a child process: it honours CUDA_VISIBLE_DEVICES as the sampler will, and this
+        # process never creates a CUDA context
         import subprocess
-        have_gpu = subprocess.run(["nvidia-smi", "-L"], capture_output=True, text=True, timeout=30).returncode == 0
+        probe = "import sys, torch; sys.exit(0 if torch.cuda.is_available() else 1)"
+        have_gpu = subprocess.run([sys.executable, "-c", probe], capture_output=True, timeout=300).returncode == 0
     except Exception:
         have_gpu = False
     note = None
@@ -536,6 +553,28 @@ def configs_leg(peak, iters=15):
     return out
 
 
+# --------------------------------------------------------------------------- outputs
+DUMP_X_BYTES = 32 << 20
+
+
+def dump_outputs(out_dir, x, eigen_estimate):
+    """--dump-outputs: x (PowerIteration.current_x, in its own dtype) and ||A x|| as .npy files.
+    An x of more than DUMP_X_BYTES is sampled: one entry from each of k equal strata of its index
+    range at a seeded offset, so every run on the same matrix size writes the same entries."""
+    import numpy as np
+    import torch
+
+    n, k = x.numel(), DUMP_X_BYTES // x.element_size()
+    if n > k:
+        lo = np.arange(k, dtype=np.int64) * n // k
+        width = np.diff(np.append(lo, n))
+        idx = lo + (np.random.default_rng(SEED).random(k) * width).astype(np.int64)
+        x = x[torch.from_numpy(idx).to(x.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "x.npy"), x.cpu().numpy())
+    np.save(os.path.join(out_dir, "eigen_estimate.npy"), np.array([eigen_estimate], dtype=np.float64))
+
+
 # --------------------------------------------------------------------------- own arm
 def own_arm(args, rank, world, local_rank):
     import numpy as np
@@ -636,6 +675,8 @@ def own_arm(args, rank, world, local_rank):
     value = 2.0 * nnz_total * args.steps / sec / 1e9
     gbs = alg_bytes_total * args.steps / sec / 1e9
     eig = it.eigen_estimate()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, it.current_x(), eig)
 
     # ---- roofline of the dominant kernel on rank 0's shard
     alg_bytes_local = local.algorithmic_bytes()

@@ -1,7 +1,8 @@
 """CPU suite: include/load.hpp (the product's Matrix Market loader + COO->CSR) against the
 reference's loader.  The expected CSR arrays in tests/golden/*.mtx.npz were produced by the
-reference's own LoadCoo + ToCsr (tests/golden/make_golden.py); where oracle/_ref exists the
-comparison is also made live on freshly written files."""
+reference's own LoadCoo + ToCsr (tests/golden/make_golden.py).  On freshly written files the
+comparison is made with the reference loader where oracle/_ref is built, else with its numpy
+restatement (tests/reference_model.py, pinned to those golden arrays in test_oracle.py)."""
 import ctypes as C
 import os
 import subprocess
@@ -11,6 +12,7 @@ import pytest
 
 from conftest import GOLDEN, ROOT
 from oracle import cpu
+import reference_model as model
 
 SHIM_SRC = os.path.join(ROOT, "tests", "cxx", "loader_shim.cpp")
 SHIM_SO = os.path.join(ROOT, "tests", "cxx", "libloader_shim.so")
@@ -80,7 +82,6 @@ def _write_random_mtx(path, n_rows, n_cols, nnz, seed, field="real", scheme="gen
     return r - 1, c - 1, v
 
 
-@pytest.mark.skipif(not cpu.have_ref(), reason="oracle/_ref not built (no /root/reference here)")
 @pytest.mark.parametrize("field,scheme", [("real", "general"), ("pattern", "general"),
                                           ("integer", "general"), ("real", "symmetric"),
                                           ("pattern", "symmetric")])
@@ -90,7 +91,7 @@ def test_random_files_match_reference_loader_live(shim, tmp_path, field, scheme)
     rc, out = load(shim, path)
     assert rc == 0, out
     n_rows, n_cols, Ap, Aj, Ax = out
-    rn, rc_, rAp, rAj, rAx = cpu.ref_load_mtx(path)
+    rn, rc_, rAp, rAj, rAx = model.original().ref_load_mtx(path)
     assert (n_rows, n_cols) == (rn, rc_)
     assert np.array_equal(Ap, rAp) and np.array_equal(Aj, rAj) and np.array_equal(Ax, rAx)
 
@@ -163,7 +164,6 @@ def _write_big_mtx(path, n, nnz, seed, field="real", scheme="general", fmt="%d %
             np.savetxt(f, np.column_stack([r, c, v]), fmt=fmt)
 
 
-@pytest.mark.skipif(not cpu.have_ref(), reason="oracle/_ref not built (no /root/reference here)")
 @pytest.mark.parametrize("threads", ["1", "3", "8"])
 @pytest.mark.parametrize("field,scheme", [("real", "general"), ("real", "symmetric"), ("pattern", "general")])
 def test_threaded_paths_match_reference_loader(shim, tmp_path, monkeypatch, field, scheme, threads):
@@ -175,7 +175,7 @@ def test_threaded_paths_match_reference_loader(shim, tmp_path, monkeypatch, fiel
     rc, out = load(shim, path)
     assert rc == 0, out
     n_rows, n_cols, Ap, Aj, Ax = out
-    rn, rc_, rAp, rAj, rAx = cpu.ref_load_mtx(path)
+    rn, rc_, rAp, rAj, rAx = model.original().ref_load_mtx(path)
     assert (n_rows, n_cols) == (rn, rc_)
     assert np.array_equal(Ap, rAp) and np.array_equal(Aj, rAj) and np.array_equal(Ax, rAx)
     # 64-bit offsets, fp64 values through the same paths
@@ -184,7 +184,6 @@ def test_threaded_paths_match_reference_loader(shim, tmp_path, monkeypatch, fiel
     assert np.array_equal(out[4].astype(np.float32), rAx)
 
 
-@pytest.mark.skipif(not cpu.have_ref(), reason="oracle/_ref not built (no /root/reference here)")
 def test_unusual_layouts_fall_back_to_the_tokenizer(shim, tmp_path, monkeypatch):
     """Two entries on one line, an entry split over two lines, trailing lines after the last
     entry: the per-line parser declines and the sequential tokenizer gives the reference's result."""
@@ -209,7 +208,7 @@ def test_unusual_layouts_fall_back_to_the_tokenizer(shim, tmp_path, monkeypatch)
         f.write("1 1 99\n2 2 99\n")             # beyond the announced count: ignored
     rc, out = load(shim, path)
     assert rc == 0, out
-    rn, rc_, rAp, rAj, rAx = cpu.ref_load_mtx(path)
+    rn, rc_, rAp, rAj, rAx = model.original().ref_load_mtx(path)
     assert np.array_equal(out[2], rAp) and np.array_equal(out[3], rAj) and np.array_equal(out[4], rAx)
 
 

@@ -2,8 +2,9 @@
 
 1. the reference's only known-answer vector (merge_based/device_spmv.cuh:95-128);
 2. golden vectors produced by the reference's own code (tests/golden/make_golden.py);
-3. where oracle/_ref exists (the build container), live bit-for-bit comparison against the
-   reference compiled from /root/reference on fresh seeded inputs.
+3. bit-for-bit comparison with the reference on fresh seeded inputs: live where oracle/_ref has
+   been built from the reference's sources, elsewhere against their numpy restatement
+   (tests/reference_model.py), itself pinned to the reference's golden vectors here.
 """
 import os
 
@@ -12,6 +13,7 @@ import pytest
 
 from conftest import GOLDEN, golden_cases, load_golden
 from oracle import cpu, generators as g
+import reference_model as model
 
 
 def test_lattice_known_answer():
@@ -103,38 +105,63 @@ def test_generators_shapes():
     assert np.array_equal(r_all[1000:1500], r_win) and np.array_equal(c_all[1000:1500], c_win)
 
 
-@pytest.mark.skipif(not cpu.have_ref(), reason="oracle/_ref not built (no /root/reference here)")
+@pytest.mark.parametrize("name", golden_cases())
+def test_numpy_restatement_matches_reference_golden(name):
+    """tests/reference_model.py reproduces every golden vector of the reference bit for bit."""
+    d = load_golden(name)
+    Ap, Aj, Ax, x = d["Ap"], d["Aj"], d["Ax"], d["x"]
+    assert np.array_equal(model.spmv(Ap, Aj, Ax, x), d["y_ref"])
+    assert np.array_equal(model.spmv_fp64(Ap, Aj, Ax, x), d["y_ref64"])
+    assert np.array_equal(model.abs_scale(Ap, Aj, Ax, x), d["abs_ref"])
+    for sr in cpu.SEMIRINGS:
+        assert np.array_equal(model.spmv_semiring(Ap, Aj, Ax, x, sr), d[f"y_{sr}"])
+    total = Ap.shape[0] - 1 + int(Ap[-1])
+    for tile in (2048, 896, 320):
+        diags = np.minimum(np.arange(d[f"coords_{tile}"].shape[0]) * tile, total)
+        got = np.array([model.merge_path_search(Ap, int(k)) for k in diags], dtype=np.int64)
+        assert np.array_equal(got, d[f"coords_{tile}"])
+    if "path_all" in d:
+        got = np.array([model.merge_path_search(Ap, k) for k in range(total + 1)], dtype=np.int64)
+        assert np.array_equal(got, d["path_all"])
+
+
+ref = model.original()
+
+
 class TestAgainstReferenceLive:
+    """The oracle against the reference on fresh inputs: `ref` is the reference itself where
+    oracle/_ref is built, else its restatement."""
+
     @pytest.mark.parametrize("seed", [1, 2, 3])
     def test_spmv_bit_exact(self, seed):
         Ap, Aj, Ax = g.ragged(3000, 900, 11.0, seed, heavy_len=4000)
         x = g.gen_x(seed, 900)
-        assert np.array_equal(cpu.spmv(Ap, Aj, Ax, x), cpu.ref_spmv(Ap, Aj, Ax, x))
-        assert np.array_equal(cpu.spmv_fp64(Ap, Aj, Ax, x), cpu.ref_spmv_fp64(Ap, Aj, Ax, x))
-        assert np.array_equal(cpu.abs_scale(Ap, Aj, Ax, x), cpu.ref_abs_scale(Ap, Aj, Ax, x))
-        y, used = cpu.ref_spmv_mt(Ap, Aj, Ax, x, 4)
-        assert np.array_equal(y, cpu.ref_spmv(Ap, Aj, Ax, x))
+        assert np.array_equal(cpu.spmv(Ap, Aj, Ax, x), ref.ref_spmv(Ap, Aj, Ax, x))
+        assert np.array_equal(cpu.spmv_fp64(Ap, Aj, Ax, x), ref.ref_spmv_fp64(Ap, Aj, Ax, x))
+        assert np.array_equal(cpu.abs_scale(Ap, Aj, Ax, x), ref.ref_abs_scale(Ap, Aj, Ax, x))
+        y, used = ref.ref_spmv_mt(Ap, Aj, Ax, x, 4)
+        assert np.array_equal(y, ref.ref_spmv(Ap, Aj, Ax, x))
         for sr in cpu.SEMIRINGS:
             assert np.array_equal(cpu.spmv_semiring(Ap, Aj, Ax, x, sr),
-                                  cpu.ref_spmv_semiring(Ap, Aj, Ax, x, sr))
+                                  ref.ref_spmv_semiring(Ap, Aj, Ax, x, sr))
 
     def test_spmv_f64_and_o64(self):
         Ap, Aj, Ax = g.ragged(1000, 300, 20.0, 5, dtype=np.float64)
         x = g.gen_x(9, 300, np.float64)
-        assert np.array_equal(cpu.spmv(Ap, Aj, Ax, x), cpu.ref_spmv(Ap, Aj, Ax, x))
+        assert np.array_equal(cpu.spmv(Ap, Aj, Ax, x), ref.ref_spmv(Ap, Aj, Ax, x))
         Ap32, Aj, Ax = g.rmat(9, 16, 4)
         x = g.gen_x(2, 512)
         Ap64 = Ap32.astype(np.int64)
-        assert np.array_equal(cpu.spmv(Ap64, Aj, Ax, x), cpu.ref_spmv(Ap64, Aj, Ax, x))
+        assert np.array_equal(cpu.spmv(Ap64, Aj, Ax, x), ref.ref_spmv(Ap64, Aj, Ax, x))
 
     def test_search_every_diagonal(self):
         Ap, _, _ = g.ragged(400, 50, 3.0, 8, heavy_len=900)
         total = Ap.shape[0] - 1 + int(Ap[-1])
         for d in range(total + 1):
-            assert cpu.merge_path_search(Ap, d) == cpu.ref_merge_path_search(Ap, d)
+            assert cpu.merge_path_search(Ap, d) == ref.ref_merge_path_search(Ap, d)
         Ap64 = Ap.astype(np.int64)
         for d in range(0, total + 1, 7):
-            assert cpu.merge_path_search(Ap64, d) == cpu.ref_merge_path_search(Ap64, d)
+            assert cpu.merge_path_search(Ap64, d) == ref.ref_merge_path_search(Ap64, d)
 
     def test_coo_to_csr(self):
         rng = np.random.default_rng(0)
@@ -142,13 +169,13 @@ class TestAgainstReferenceLive:
         cols = rng.integers(0, 70, 2000).astype(np.int32)
         vals = rng.uniform(-1, 1, 2000).astype(np.float32)
         a = cpu.coo_to_csr(50, rows, cols, vals)
-        b = cpu.ref_coo_to_csr(50, 70, rows, cols, vals)
+        b = ref.ref_coo_to_csr(50, 70, rows, cols, vals)
         for u, v in zip(a, b):
             assert np.array_equal(u, v)
 
     def test_loader_fixtures_match_reference(self):
         for f in ("general_real.mtx", "symmetric_pattern.mtx", "symmetric_integer.mtx"):
-            n_rows, n_cols, Ap, Aj, Ax = cpu.ref_load_mtx(os.path.join(GOLDEN, f))
+            n_rows, n_cols, Ap, Aj, Ax = ref.ref_load_mtx(os.path.join(GOLDEN, f))
             d = np.load(os.path.join(GOLDEN, f + ".npz"))
             assert n_rows == int(d["n_rows"]) and n_cols == int(d["n_cols"])
             assert np.array_equal(Ap, d["Ap"]) and np.array_equal(Aj, d["Aj"])
