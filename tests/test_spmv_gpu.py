@@ -142,6 +142,17 @@ def _csr(lens, n_cols, seed=0, dtype=np.float32, off=np.int32):
     return Ap.astype(off), Aj, Ax
 
 
+def _tile(tma=False):
+    """Path items per tile of the merge kernel (tma: of the TMA-staged variant)."""
+    from spmv_samples_b200 import _lib, spmv
+    old = spmv.get_option("merge_staging")
+    spmv.set_option("merge_staging", 1 if tma else 0)
+    try:
+        return int(_lib.lib().spmvb200_merge_tile_items(32, 32))
+    finally:
+        spmv.set_option("merge_staging", old)
+
+
 EDGE = {
     "all_rows_empty": lambda: _csr([0] * 777, 10),
     "single_row_single_nnz": lambda: _csr([1], 5),
@@ -150,10 +161,15 @@ EDGE = {
     "all_nnz_in_last_row": lambda: _csr([0] * 5000 + [7777], 100),
     "all_nnz_in_first_row": lambda: _csr([7777] + [0] * 5000, 100),
     "nnz_not_multiple_of_4": lambda: _csr([3, 1, 2, 5, 0, 7, 1], 9),
-    "exact_tile_multiple": lambda: _csr([15] * 128, 64),          # 128 rows + 1920 nnz = 2048
-    "tile_boundary_on_row_end": lambda: _csr([2047] + [2047], 64),
+    # T = the default merge kernel's tile (1020 path items = rows + nonzeros), T_tma = the
+    # TMA-staged variant's (2044), both as the library reports them
+    "exact_tile_multiple": lambda: _csr([_tile() // 17 - 1] * 17, 64),    # 17 rows + 17 * 59 nnz = 1020
+    "exact_tile_multiple_tma": lambda: _csr([_tile(tma=True) // 4 - 1] * 4, 64),   # 4 + 4 * 510 = 2044
+    "tile_boundary_on_row_end": lambda: _csr([_tile() - 1] * 2, 64),     # row ends at items T-1, 2T-1
+    "tile_boundary_on_row_end_tma": lambda: _csr([_tile(tma=True) - 1] * 2, 64),
     "n_cols_1": lambda: _csr([1, 0, 1, 1, 0] * 50, 1),
-    "two_tiles_one_row_each": lambda: _csr([2047, 2047, 1], 33),
+    "two_tiles_one_row_each": lambda: _csr([_tile() - 1] * 2 + [1], 33),
+    "two_tiles_one_row_each_tma": lambda: _csr([_tile(tma=True) - 1] * 2 + [1], 33),
     "long_rows_f64": lambda: _csr([4099, 1, 4097, 0, 8191], 512, dtype=np.float64),
     "o64_mixed": lambda: _csr([5, 0, 300, 2, 2, 9000, 1], 700, off=np.int64),
 }
