@@ -180,6 +180,43 @@ typedef struct {
 } spmvb200_spmm_args_t;
 SPMVB200_API int spmvb200_spmm(const spmvb200_spmm_args_t *args);
 
+/* ---- conjugate-gradient solve A x = b on the device (csrc/cg.cu) ---------------------------
+ * A is n x n, symmetric positive definite, in CSR; preconditioned CG (Hestenes-Stiefel) with
+ * M = I, or M = diag(A) with SPMVB200_CG_JACOBI.  One iteration is one SpMV of `kind` (any kind
+ * spmvb200_spmv accepts; SPMVB200_FLAG_STATIC_PATTERN on every call after the first) and three
+ * streaming kernels.  Dot products accumulate in double in a fixed order, so a solve is
+ * deterministic for the deterministic kinds.  Stops after the first iteration with
+ * ||r|| <= rtol * ||b|| (r the recursive residual), after max_iter iterations, or at a breakdown
+ * (p.q <= 0 or not finite: A is not SPD); a breakdown is not an error.  x holds the initial guess
+ * on entry and the solution on return; b = 0 gives x = 0.  residual_norm is ||b - A x|| of the
+ * returned x, computed once more in fp64.  The host reads the device flags once per batch of
+ * iterations (1, 2, 4, ... 64), not per iteration.  Enqueued on `stream`; synchronises before it
+ * returns.  Workspace (3 vectors, 5 with Jacobi) is cached per (device, stream) like the other
+ * scratch and freed by spmvb200_release_cache.  Errors: SPMVB200_ERR_INVALID for an unknown kind
+ * or flag, rtol <= 0 or NaN, max_iter < 0, a NULL pointer with n > 0, x == b, or (Jacobi) a row
+ * whose diagonal entry is missing or zero; the alignment rules of spmvb200_spmv. */
+#define SPMVB200_CG_JACOBI 1
+typedef struct {
+    int32_t kind, offset_bits, value_bits, flags; /* flags: 0 or SPMVB200_CG_JACOBI */
+    int64_t n, nnz;                               /* A is n x n */
+    const void *Ap;
+    const int32_t *Aj;
+    const void *Ax;
+    const void *b;
+    void *x; /* initial guess in, solution out (DEVICE) */
+    double rtol;
+    int64_t max_iter;
+    spmvb200_stream_t stream;
+} spmvb200_cg_args_t;
+typedef struct {
+    int64_t iterations;
+    double residual_norm;
+    double b_norm;
+    int32_t converged;
+    int32_t breakdown;
+} spmvb200_cg_result_t;
+SPMVB200_API int spmvb200_cg(const spmvb200_cg_args_t *args, spmvb200_cg_result_t *out);
+
 /* ---- merge-path partition, exposed so parity tests can demand bit-exact coordinates --- */
 /* Row coordinate of the merge path on each diagonal min(t * tile_items, n_rows + nnz),
  * t = 0 .. n_coords-1, written to the DEVICE array coords_x (int32).  The nonzero

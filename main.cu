@@ -20,6 +20,9 @@
 //   default does, through option "assume_static_pattern": partition and hot-x plan are reused)
 //   --power K [--gpus N]: K power-iteration steps, the matrix row-sharded over N GPUs of the box
 //   (one process, peer access; csrc/multi.cu) -- the multi-GPU configuration without Python
+//   --cg RTOL [--jacobi]: for a square matrix, b = A*1 and x0 = 0, then one conjugate-gradient solve
+//   (Jacobi-preconditioned with --jacobi) per kind through spmvb200_cg; exits non-zero if one does
+//   not converge
 #include <algorithm>
 #include <chrono>
 #include <cmath>
@@ -55,6 +58,8 @@ struct Options {
     uint64_t seed = 0x5EEDB200ull;
     int gpus = 1;    // --gpus N: the row-sharded power iteration over N GPUs of this box
     int power = 0;   // --power K: K power-iteration steps x <- A x / ||A x|| (BASELINE.json configs[4])
+    double cg_rtol = 0;      // --cg RTOL: one CG solve of A x = A*1 per kind
+    bool cg_jacobi = false;  // --jacobi: with M = diag(A)
 };
 
 template <typename T>
@@ -62,6 +67,92 @@ static T *device_alloc(size_t n) {
     T *p = nullptr;
     checkCudaErr(cudaMalloc((void **)&p, std::max<size_t>(n, 1) * sizeof(T)));
     return p;
+}
+
+// the SpMV kind behind a label of the kind table (include/spmv.h), or -1
+static int kind_id(const string &k) {
+    if (k == "merge" || k == "cub_merge" || k == "merge_genl") return SPMVB200_KIND_MERGE;
+    if (k == "vector" || k == "cusp" || k == "cusp1" || k == "cusp2") return SPMVB200_KIND_VECTOR;
+    if (k == "light" || k == "light_vec" || k == "light_warp") return SPMVB200_KIND_LIGHT;
+    if (k == "stream") return SPMVB200_KIND_STREAM;
+    if (k == "auto") return SPMVB200_KIND_AUTO;
+    if (k == "cusparse") return SPMVB200_KIND_CUSPARSE;
+    return -1;
+}
+
+// --cg: b = A*1, x0 = 0, one solve per kind; returns the number of kinds that did not converge
+template <typename offset_t, typename value_t>
+static int run_cg(const Options &opt, index_t n, offset_t nnz, offset_t *dAp, index_t *dAj, value_t *dAx) {
+    const size_t vb = sizeof(value_t);
+    vector<value_t> ones((size_t)n, value_t(1)), hx((size_t)n);
+    value_t *d1 = device_alloc<value_t>((size_t)n), *dB = device_alloc<value_t>((size_t)n);
+    value_t *dX = device_alloc<value_t>((size_t)n);
+    checkCudaErr(cudaMemcpy(d1, ones.data(), (size_t)n * vb, cudaMemcpyHostToDevice));
+    spmvb200_args_t s;
+    memset(&s, 0, sizeof(s));
+    s.kind = SPMVB200_KIND_MERGE;
+    s.offset_bits = sizeof(offset_t) * 8;
+    s.value_bits = vb * 8;
+    s.n_rows = s.n_cols = n;
+    s.nnz = (int64_t)nnz;
+    s.Ap = dAp;
+    s.Aj = dAj;
+    s.Ax = dAx;
+    s.x = d1;
+    s.y = dB;
+    checkSpmvStatus(spmvb200_spmv(&s));
+    checkCudaErr(cudaDeviceSynchronize());
+    cudaEvent_t e0, e1;
+    checkCudaErr(cudaEventCreate(&e0));
+    checkCudaErr(cudaEventCreate(&e1));
+    printf("Conjugate gradients (b = A*1, x0 = 0, rtol %.1e%s, max %d iterations):\n", opt.cg_rtol,
+           opt.cg_jacobi ? ", Jacobi preconditioner" : "", n);
+    int failures = 0;
+    for (const auto &kind : opt.kinds) {
+        const int id = kind_id(kind);
+        if (id < 0) {
+            printf("[%-12s] no such kind\n", kind.data());
+            ++failures;
+            continue;
+        }
+        checkCudaErr(cudaMemset(dX, 0, (size_t)n * vb));
+        spmvb200_cg_args_t a;
+        memset(&a, 0, sizeof(a));
+        a.kind = id;
+        a.offset_bits = sizeof(offset_t) * 8;
+        a.value_bits = vb * 8;
+        a.flags = opt.cg_jacobi ? SPMVB200_CG_JACOBI : 0;
+        a.n = n;
+        a.nnz = (int64_t)nnz;
+        a.Ap = dAp;
+        a.Aj = dAj;
+        a.Ax = dAx;
+        a.b = dB;
+        a.x = dX;
+        a.rtol = opt.cg_rtol;
+        a.max_iter = n;
+        spmvb200_cg_result_t r;
+        checkCudaErr(cudaEventRecord(e0, nullptr));
+        checkSpmvStatus(spmvb200_cg(&a, &r));  // synchronises
+        checkCudaErr(cudaEventRecord(e1, nullptr));
+        checkCudaErr(cudaEventSynchronize(e1));
+        float ms = 0.f;
+        checkCudaErr(cudaEventElapsedTime(&ms, e0, e1));
+        checkCudaErr(cudaMemcpy(hx.data(), dX, (size_t)n * vb, cudaMemcpyDeviceToHost));
+        double err = 0.0;
+        for (index_t i = 0; i < n; ++i) err = std::max(err, std::abs((double)hx[(size_t)i] - 1.0));
+        failures += !r.converged;
+        printf("[%-12s] %lld iterations  |b-Ax|/|b| = %.3e  max|x-1| = %.3e  %.3f ms  %.4f ms/iteration  %s\n",
+               kind.data(), (long long)r.iterations, r.b_norm > 0 ? r.residual_norm / r.b_norm : r.residual_norm, err,
+               ms, r.iterations ? ms / r.iterations : 0.0,
+               r.converged ? "CONVERGED" : r.breakdown ? "BREAKDOWN" : "NOT CONVERGED");
+    }
+    checkCudaErr(cudaEventDestroy(e0));
+    checkCudaErr(cudaEventDestroy(e1));
+    checkCudaErr(cudaFree(d1));
+    checkCudaErr(cudaFree(dB));
+    checkCudaErr(cudaFree(dX));
+    return failures;
 }
 
 template <typename offset_t, typename value_t>
@@ -200,6 +291,15 @@ static int run(const Options &opt, const string &name, index_t n_rows, index_t n
         spmvb200_power_destroy(pw);
     }
 
+    if (opt.cg_rtol > 0) {
+        if (n_rows == n_cols) {
+            failures += run_cg<offset_t, value_t>(opt, n_rows, nnz, dA_csrOffsets, dA_columns, dA_values);
+        } else {
+            printf("Conjugate gradients: the matrix is not square\n");
+            ++failures;
+        }
+    }
+
     if (flush_buf) checkCudaErr(cudaFree(flush_buf));
     checkCudaErr(cudaFree(dX));
     checkCudaErr(cudaFree(dY));
@@ -290,7 +390,7 @@ static int run_synthetic(const Options &opt, const string &cfg, long size) {
 int main(int argc, char **argv) {
     if (argc < 3) {
         cerr << "usage: ./bin/<program-name>  <filename.mtx | synthetic:c1..c5[:size]>  <SpMV_kind_string>..."
-                "  [--iters N] [--x ones|random] [--flush] [--dynamic-pattern] [--peak GB/s] [--power K [--gpus N]]"
+                "  [--iters N] [--x ones|random] [--flush] [--dynamic-pattern] [--peak GB/s] [--power K [--gpus N]] [--cg RTOL [--jacobi]]"
              << endl;
         exit(1);
     }
@@ -305,6 +405,8 @@ int main(int argc, char **argv) {
         else if (a == "--peak" && i + 1 < argc) opt.peak_gbs = atof(argv[++i]);
         else if (a == "--gpus" && i + 1 < argc) opt.gpus = atoi(argv[++i]);
         else if (a == "--power" && i + 1 < argc) opt.power = atoi(argv[++i]);
+        else if (a == "--cg" && i + 1 < argc) opt.cg_rtol = atof(argv[++i]);
+        else if (a == "--jacobi") opt.cg_jacobi = true;
         else opt.kinds.push_back(a);
     }
     if (opt.kinds.empty() || opt.iters < 1) {

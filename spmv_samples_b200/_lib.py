@@ -17,6 +17,7 @@ CSRC = os.path.join(_PKG, "csrc")
 OK = 0
 KIND_MERGE, KIND_VECTOR, KIND_LIGHT, KIND_AUTO, KIND_CUSPARSE, KIND_STREAM = 0, 1, 2, 3, 4, 5
 FLAG_STATIC_PATTERN = 1   # SPMVB200_FLAG_STATIC_PATTERN
+CG_JACOBI = 1             # SPMVB200_CG_JACOBI
 SEMIRINGS = {"plus_times": 0, "min_plus": 1, "max_plus": 2, "or_and": 3}
 MAX_PEERS = 8
 IPC_HANDLE_BYTES = 64
@@ -47,6 +48,22 @@ class SpmmArgs(C.Structure):
         ("Ap", C.c_void_p), ("Aj", C.c_void_p), ("Ax", C.c_void_p), ("X", C.c_void_p),
         ("ldx", C.c_int64), ("Y", C.c_void_p), ("ldy", C.c_int64), ("alpha_dev", C.c_void_p),
         ("stream", C.c_void_p),
+    ]
+
+
+class CgArgs(C.Structure):
+    _fields_ = [
+        ("kind", C.c_int32), ("offset_bits", C.c_int32), ("value_bits", C.c_int32), ("flags", C.c_int32),
+        ("n", C.c_int64), ("nnz", C.c_int64),
+        ("Ap", C.c_void_p), ("Aj", C.c_void_p), ("Ax", C.c_void_p), ("b", C.c_void_p), ("x", C.c_void_p),
+        ("rtol", C.c_double), ("max_iter", C.c_int64), ("stream", C.c_void_p),
+    ]
+
+
+class CgOut(C.Structure):
+    _fields_ = [
+        ("iterations", C.c_int64), ("residual_norm", C.c_double), ("b_norm", C.c_double),
+        ("converged", C.c_int32), ("breakdown", C.c_int32),
     ]
 
 
@@ -86,6 +103,8 @@ def lib() -> C.CDLL:
     L.spmvb200_spmv.restype = C.c_int
     L.spmvb200_spmm.argtypes = [C.POINTER(SpmmArgs)]
     L.spmvb200_spmm.restype = C.c_int
+    L.spmvb200_cg.argtypes = [C.POINTER(CgArgs), C.POINTER(CgOut)]
+    L.spmvb200_cg.restype = C.c_int
     L.spmvb200_launch_count.restype = C.c_int64
     L.spmvb200_get_option.restype = C.c_int64
     L.spmvb200_get_option.argtypes = [C.c_char_p]

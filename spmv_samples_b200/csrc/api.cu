@@ -165,6 +165,31 @@ int spmvb200_spmm(const spmvb200_spmm_args_t *a) {
     return SPMVB200_ERR_UNSUPPORTED;
 }
 
+// ---- conjugate gradients -------------------------------------------------------------------
+// Every argument is checked here, before any CUDA call (so also without a device).
+int spmvb200_cg(const spmvb200_cg_args_t *a, spmvb200_cg_result_t *out) {
+    if (!a || !out) return SPMVB200_ERR_INVALID;
+    if (a->kind < SPMVB200_KIND_MERGE || a->kind > SPMVB200_KIND_STREAM) return SPMVB200_ERR_INVALID;
+    if (a->flags & ~SPMVB200_CG_JACOBI) return SPMVB200_ERR_INVALID;
+    if (!(a->rtol > 0.0) || a->max_iter < 0 || a->n < 0 || a->nnz < 0) return SPMVB200_ERR_INVALID;
+    if ((a->offset_bits != 32 && a->offset_bits != 64) || (a->value_bits != 32 && a->value_bits != 64))
+        return SPMVB200_ERR_UNSUPPORTED;
+    if (a->n > 0x7fffffffLL) return SPMVB200_ERR_INVALID;
+    if (a->offset_bits == 32 && a->nnz > 0x7fffffffLL - 4096) return SPMVB200_ERR_UNSUPPORTED;
+    if (a->n == 0) {
+        std::memset(out, 0, sizeof(*out));
+        out->converged = 1;
+        return SPMVB200_OK;
+    }
+    if (!a->Ap || !a->b || !a->x || (a->nnz > 0 && (!a->Aj || !a->Ax))) return SPMVB200_ERR_INVALID;
+    if (a->x == a->b) return SPMVB200_ERR_INVALID;
+    if (!aligned16(a->Ap) || !aligned16(a->Aj) || !aligned16(a->Ax)) return SPMVB200_ERR_ALIGNMENT;
+    if (a->offset_bits == 32 && a->value_bits == 32) return cg_solve<int32_t, float>(*a, out);
+    if (a->offset_bits == 32 && a->value_bits == 64) return cg_solve<int32_t, double>(*a, out);
+    if (a->offset_bits == 64 && a->value_bits == 32) return cg_solve<int64_t, float>(*a, out);
+    return cg_solve<int64_t, double>(*a, out);
+}
+
 // ---- partition / row split -----------------------------------------------------------------
 int spmvb200_merge_path_partition_o32(int32_t n_rows, int32_t nnz, const int32_t *Ap,
                                       int64_t tile_items, int64_t n_coords, int32_t *coords_x,
