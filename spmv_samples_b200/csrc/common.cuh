@@ -60,7 +60,7 @@ int apply_carveout(const void *kernel, int64_t percent);
 // Slots keep independent buffers so a kernel can hold several at once.
 enum ScratchSlot { SCRATCH_COORDS = 0, SCRATCH_CARRY_ROW, SCRATCH_CARRY_VAL, SCRATCH_COUNTER,
                    SCRATCH_STATS, SCRATCH_MISC, SCRATCH_SPMM_X, SCRATCH_SPMM_Y, SCRATCH_XHOT, SCRATCH_NORM,
-                   SCRATCH_CG, SCRATCH_NUM_SLOTS };
+                   SCRATCH_CG, SCRATCH_ROW_END, SCRATCH_START_MASK, SCRATCH_NUM_SLOTS };
 int scratch_get(cudaStream_t stream, ScratchSlot slot, size_t bytes, void **out);
 
 // What the last merge-path partition launched on a (device, stream) wrote, and where: lets a
@@ -75,6 +75,11 @@ struct PartitionTag {
 };
 bool partition_tag_matches(cudaStream_t stream, const PartitionTag &tag);
 void partition_tag_store(cudaStream_t stream, const PartitionTag &tag);
+// The persistent merge kernel's tile descriptors (merge.cu) are derived from the coordinates of the
+// last partition on a (device, stream); a new search makes them stale.  tile_desc_current: the
+// descriptors at (row_end, start_mask) were built from those coordinates.
+bool tile_desc_current(cudaStream_t stream, const void *row_end, const void *start_mask);
+void tile_desc_store(cudaStream_t stream, const void *row_end, const void *start_mask);
 void scratch_release_all();
 
 int64_t option_get(const char *name, int64_t fallback);

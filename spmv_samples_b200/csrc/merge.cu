@@ -320,17 +320,45 @@ template <> struct __align__(16) WarpTotal<double> { double val; int rid; int pa
 template <int BLOCK, typename ValT>
 struct __align__(16) TileSmem {
     ValT scan[BLOCK * kMergeIPT];
-    // row-start flags, one byte per slot.  (One BIT per slot, set with atomicOr, saves 1.8 KB per
-    // 256-thread CTA and fits one more CTA per SM inside the 64 KB carveout, but measured slower:
-    // R-MAT scale 24 1146 -> 1166 us, scale 27 14.70 -> 14.93 ms.)
-    unsigned char flag[BLOCK * kMergeIPT];
     WarpTotal<ValT> w[BLOCK / 32];
 };
 
+// Tile descriptors of the persistent kernel, built once per partition by tile_desc_kernel:
+//   row_end[r]  = Ap[r+1] - sy(t), t the tile in which row r's end item lies (<= TILE: 16 bits);
+//   start_mask  = 1 bit per slot and tile, bit s of tile t set iff a row starts at slot s -- the
+//                 byte flags that the scatter of Ap writes in the GROUPS == 1 body.
+struct TileDesc {
+    const uint16_t *row_end;
+    const unsigned char *start_mask;
+};
+// Only the persistent fp32 kernel with 64-bit offsets uses them: there they are about half the bytes of
+// Ap (2 B per row + 128 B per tile against 8 B per row; R-MAT scale 27: 0.55 against 1.07 GB per
+// SpMV).  With 32-bit offsets they are as many bytes as Ap, and the kernel that used them (and its
+// coordinates one tile ahead) measured slower: R-MAT scale 24, static pattern, 994 -> 1031 us per SpMV.
+// descriptor loads: read once per SpMV, so they bypass the L1 and go first out of the L2, where they
+// would otherwise push out lines of x (R-MAT scale 27: step 10.78 with plain loads, 10.62 ms with these)
+__device__ __forceinline__ unsigned ldg_stream_u8(const unsigned char *p, uint64_t policy) {
+    unsigned v;
+    asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.u8 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(policy));
+    return v;
+}
+__device__ __forceinline__ int ldg_stream_u16(const uint16_t *p, uint64_t policy) {
+    unsigned v;
+    asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.u16 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(policy));
+    return (int)v;
+}
+// fp64 (off by default in the table kernel) keeps Ap as well: its body spills with the descriptors.
+template <int GROUPS, typename OffT, typename ValT> constexpr bool tile_desc_used() {
+    return GROUPS > 1 && sizeof(OffT) == 8 && sizeof(ValT) == 4;
+}
+
 // GROUPS == 1: the CTA is one tile (tile = blockIdx.x, static shared memory, __syncthreads).
 // GROUPS > 1 (merge_tile_table_kernel): the CTA is GROUPS independent groups of BLOCK threads, each
-// working on its own tile out of its own TileSmem with its own named barrier, and `table` holds
-// the x values of ranks 0 .. table_n-1 of the hot-x plan in shared memory.
+// working on its own tile out of its own TileSmem and flags with its own named barrier, and `table`
+// holds the x values of ranks 0 .. table_n-1 of the hot-x plan in shared memory.
+// DESC (tile_desc_used): the caller passes the tile's coordinates (sx, ex), and the row ends and row
+// starts come from the tile descriptors: no load of Ap, no flags, no flag scatter and two barriers
+// per tile instead of four.  Otherwise the row ends come from Ap.
 template <int BLOCK, int HAS_PEERS, bool HOT, int GROUPS, typename OffT, typename ValT>
 __device__ __forceinline__ void
 merge_tile_reg_body(int32_t n_rows, OffT nnz, const OffT *__restrict__ Ap,
@@ -340,17 +368,24 @@ merge_tile_reg_body(int32_t n_rows, OffT nnz, const OffT *__restrict__ Ap,
                     const int32_t *__restrict__ coords_x, int32_t *__restrict__ carry_row,
                     ValT *__restrict__ carry_val, const ValT *__restrict__ x_hot_biased,
                     int64_t tile_of_group = 0, TileSmem<BLOCK, ValT> *group_smem = nullptr,
-                    const ValT *table = nullptr, uint32_t table_n = 0) {
+                    const ValT *table = nullptr, uint32_t table_n = 0, unsigned char *group_flag = nullptr,
+                    int32_t group_sx = 0, int32_t group_ex = 0, TileDesc desc = {}) {
     constexpr int IPT = kMergeIPT;
     constexpr int SLOTS = BLOCK * IPT;
     constexpr int TILE = SLOTS - 4;  // path items per tile
+    constexpr bool DESC = tile_desc_used<GROUPS, OffT, ValT>();
     TileSmem<BLOCK, ValT> *sm = group_smem;
+    unsigned char *s_flag = group_flag;
     if constexpr (GROUPS == 1) {
         __shared__ TileSmem<BLOCK, ValT> s_cta;
+        // row-start flags, one byte per slot.  (One BIT per slot, set with atomicOr, saves 1.8 KB per
+        // 256-thread CTA and fits one more CTA per SM inside the 64 KB carveout, but measured slower:
+        // R-MAT scale 24 1146 -> 1166 us, scale 27 14.70 -> 14.93 ms.)
+        __shared__ __align__(16) unsigned char s_cta_flag[SLOTS];
         sm = &s_cta;
+        s_flag = s_cta_flag;
     }
     ValT *const s_scan = sm->scan;
-    unsigned char *const s_flag = sm->flag;
     WarpTotal<ValT> *const s_w = sm->w;
     const int grp = GROUPS == 1 ? 0 : (int)(threadIdx.x / BLOCK);
     auto tile_sync = [grp]() {
@@ -363,15 +398,29 @@ merge_tile_reg_body(int32_t n_rows, OffT nnz, const OffT *__restrict__ Ap,
     const int64_t total = (int64_t)n_rows + (int64_t)nnz;
     const int64_t d0 = tile * TILE;
     const int64_t d1 = d0 + TILE < total ? d0 + TILE : total;
-    const int32_t sx = __ldg(coords_x + tile);
-    const int32_t ex = __ldg(coords_x + tile + 1);
+    const int32_t sx = DESC ? group_sx : __ldg(coords_x + tile);
+    const int32_t ex = DESC ? group_ex : __ldg(coords_x + tile + 1);
     const int64_t sy = d0 - sx;
     const int R = ex - sx;                // rows that end inside this tile
     const int Z = (int)((d1 - ex) - sy);  // nonzeros inside this tile
     const int shift = (int)(sy & 3);      // slot s holds tile-local nonzero s - shift
     const int64_t a0 = sy - shift;        // 16-byte aligned position of slot 0 in Aj / Ax
 
-    *reinterpret_cast<uint2 *>(s_flag + tid * IPT) = make_uint2(0u, 0u);
+    if constexpr (!DESC) *reinterpret_cast<uint2 *>(s_flag + tid * IPT) = make_uint2(0u, 0u);
+
+    // ---- DESC: this thread's byte of the start mask (its 8 slots' row-start bits), and the
+    // row ends of its first row (q0) and of the row before (b0), issued with the Aj / Ax loads so that
+    // they have arrived when the scan ends.  Row sx's nonzeros start at or before sy (the merge path
+    // has Ap[sx] <= sy), hence b = 0 for j = 0.
+    unsigned mask_byte = 0;
+    int q0 = 0, b0 = 0;
+    if constexpr (DESC) {
+        const uint64_t pol_desc = policy_evict_first();
+        mask_byte = ldg_stream_u8(desc.start_mask + tile * (SLOTS / 8) + tid, pol_desc);
+        if (tid < R) q0 = ldg_stream_u16(desc.row_end + sx + tid, pol_desc);
+        // lanes 1..31 take b0 from the lane below after the gathers; lane 0 loads its own
+        if ((tid & 31) == 0 && tid > 0 && tid < R) b0 = ldg_stream_u16(desc.row_end + sx + tid - 1, pol_desc);
+    }
 
     // ---- this thread's 8 consecutive slots straight into registers
     const int slot0 = tid * IPT;
@@ -403,12 +452,13 @@ merge_tile_reg_body(int32_t n_rows, OffT nnz, const OffT *__restrict__ Ap,
         }
     }
     const ValT alpha = alpha_dev ? __ldg(alpha_dev) : (ValT)1;
-    tile_sync();  // flags are clear
-
-    // ---- row-start flags, one thread per row end (Ap read coalesced, no staging)
-    for (int j = tid; j < R; j += BLOCK) {
-        const int64_t q = (int64_t)__ldg(Ap + sx + 1 + j) - sy;
-        if (q < Z) s_flag[(int)q + shift] = 1;
+    if constexpr (!DESC) {
+        tile_sync();  // flags are clear
+        // ---- row-start flags, one thread per row end (Ap read coalesced, no staging)
+        for (int j = tid; j < R; j += BLOCK) {
+            const int64_t q = (int64_t)__ldg(Ap + sx + 1 + j) - sy;
+            if (q < Z) s_flag[(int)q + shift] = 1;
+        }
     }
     // ---- x gathers, all eight issued before the first use
     {
@@ -432,15 +482,23 @@ merge_tile_reg_body(int32_t n_rows, OffT nnz, const OffT *__restrict__ Ap,
             p[k] = (i >= 0 && i < Z) ? p[k] * xv[k] : (ValT)0;
         }
     }
-    tile_sync();  // flags are set
-
-    // ---- segmented scan (as in the TMA variant)
-    const uint2 fw = *reinterpret_cast<const uint2 *>(s_flag + slot0);
-    const unsigned long long fbits = ((unsigned long long)fw.y << 32) | fw.x;
+    if constexpr (DESC) {   // the row end before this thread's first row: the lane below's q0
+        const int up = __shfl_up_sync(0xffffffffu, q0, 1);
+        if ((tid & 31) != 0) b0 = up;
+    }
+    // ---- segmented scan (as in the TMA variant).  The flag of slot k is bit FS * k of fbits: the
+    // bytes of the shared flags or the bits of the start mask (DESC).
+    constexpr int FS = DESC ? 1 : 8;
+    unsigned long long fbits = mask_byte;
+    if constexpr (!DESC) {
+        tile_sync();  // flags are set
+        const uint2 fw = *reinterpret_cast<const uint2 *>(s_flag + slot0);
+        fbits = ((unsigned long long)fw.y << 32) | fw.x;
+    }
     int flag = fbits != 0ull;
     ValT val = (ValT)0;
 #pragma unroll
-    for (int k = 0; k < IPT; ++k) val = ((fbits >> (8 * k)) & 1ull) ? p[k] : val + p[k];
+    for (int k = 0; k < IPT; ++k) val = ((fbits >> (FS * k)) & 1ull) ? p[k] : val + p[k];
     const int lane = tid & 31, warp = tid >> 5;
     // the row-start bits of the warp as one ballot: lane L's sum reaches back to lane L - d iff
     // none of lanes L - d + 1 .. L holds a flag -- 6 shuffles per thread instead of 12
@@ -469,7 +527,7 @@ merge_tile_reg_body(int32_t n_rows, OffT nnz, const OffT *__restrict__ Ap,
     ValT run = ef ? ev : wv + ev;
 #pragma unroll
     for (int k = 0; k < IPT; ++k) {
-        run = ((fbits >> (8 * k)) & 1ull) ? p[k] : run + p[k];
+        run = ((fbits >> (FS * k)) & 1ull) ? p[k] : run + p[k];
         p[k] = run;
     }
     sts8(s_scan + slot0, p);
@@ -479,9 +537,18 @@ merge_tile_reg_body(int32_t n_rows, OffT nnz, const OffT *__restrict__ Ap,
     // Row sx+j covers tile-local nonzeros [max(Ap[sx+j]-sy, 0), Ap[sx+j+1]-sy).
     const ValT *scan = s_scan + shift;
     for (int j = tid; j < R; j += BLOCK) {
-        const int64_t b64 = (int64_t)__ldg(Ap + sx + j) - sy;
-        const int q = (int)((int64_t)__ldg(Ap + sx + 1 + j) - sy);
-        const int b = b64 > 0 ? (int)b64 : 0;
+        int q, b;
+        if constexpr (!DESC) {
+            const int64_t b64 = (int64_t)__ldg(Ap + sx + j) - sy;
+            q = (int)((int64_t)__ldg(Ap + sx + 1 + j) - sy);
+            b = b64 > 0 ? (int)b64 : 0;
+        } else if (j == tid) {
+            q = q0;
+            b = b0;
+        } else {  // more than BLOCK rows end in the tile (runs of empty rows)
+            q = __ldg(desc.row_end + sx + j);
+            b = __ldg(desc.row_end + sx + j - 1);
+        }
         const ValT sum = q > b ? scan[q - 1] : (ValT)0;
         // the peer fan-out is compiled in only when there are peers: its code cost the
         // (o32, fp32) kernel its 32-register budget (spills; c3 1224 -> 1459 us)
@@ -495,9 +562,14 @@ merge_tile_reg_body(int32_t n_rows, OffT nnz, const OffT *__restrict__ Ap,
         } else {
             y[(int64_t)sx + j] = alpha * sum;
         }
+        if (DESC && j == R - 1) {  // the tile's last row end is in hand: carry out what follows it
+            carry_row[tile] = ex;
+            carry_val[tile] = Z > q ? scan[Z - 1] : (ValT)0;
+        }
     }
-    if (tid == 0) {
-        const int64_t lq = R > 0 ? (int64_t)__ldg(Ap + ex) - sy : 0;
+    if (tid == 0 && (!DESC || R == 0)) {
+        // nonzeros after the last row end of the tile belong to row ex: carry them out
+        const int64_t lq = !DESC && R > 0 ? (int64_t)__ldg(Ap + ex) - sy : 0;
         const int lastq = lq > 0 ? (int)lq : 0;
         carry_row[tile] = ex;
         carry_val[tile] = Z > lastq ? scan[Z - 1] : (ValT)0;
@@ -756,7 +828,10 @@ merge_tile_hot_kernel(MERGE_REG_KERNEL_ARGS, const ValT *__restrict__ x_hot_bias
 //   scale 27 (hot-x plan + table): 11.4 ms -> 10.9 persistent -> 10.4 with 15 K columns (15 %).
 // The table takes its space from the L1, which is what holds the gathers in flight; the sizes
 // are chosen in launch_merge ("hot_x_table_bytes").  The tile body is the flag form's, with
-// group-local barriers; products and their order are unchanged.
+// group-local barriers; products and their order are unchanged.  The partition is fixed while the
+// kernel is reused, so with 64-bit offsets and fp32 its row ends and row starts are read from tile
+// descriptors built once with it (TileDesc) instead of from Ap, and each group loads its next
+// tile's coordinates a tile ahead.
 #ifndef SPMV_TABLE_GROUPS
 #define SPMV_TABLE_GROUPS 8
 #endif
@@ -769,21 +844,67 @@ constexpr int kTableBlock = 128;
 template <int HAS_PEERS, typename OffT, typename ValT>
 __global__ void __launch_bounds__(kTableGroups *kTableBlock, kTableCtas)
 merge_tile_table_kernel(MERGE_REG_KERNEL_ARGS, const ValT *__restrict__ x_hot_biased,
-                        const ValT *__restrict__ x_hot, uint32_t table_n, int64_t num_tiles) {
+                        const ValT *__restrict__ x_hot, uint32_t table_n, int64_t num_tiles, TileDesc desc) {
+    constexpr bool DESC = tile_desc_used<kTableGroups, OffT, ValT>();
     extern __shared__ __align__(128) unsigned char smem_raw[];
     using Smem = TileSmem<kTableBlock, ValT>;
     Smem *const groups = reinterpret_cast<Smem *>(smem_raw);
-    ValT *const table = reinterpret_cast<ValT *>(smem_raw + sizeof(Smem) * kTableGroups);
+    unsigned char *const flags = smem_raw + sizeof(Smem) * kTableGroups;   // without descriptors
+    ValT *const table = reinterpret_cast<ValT *>(flags + (DESC ? 0 : kTableGroups * kTableBlock * kMergeIPT));
     for (uint32_t i = threadIdx.x; i < table_n; i += kTableGroups * kTableBlock) table[i] = __ldg(x_hot + i);
     __syncthreads();
     const int grp = (int)(threadIdx.x / kTableBlock);
-    for (int64_t tile = (int64_t)blockIdx.x * kTableGroups + grp; tile < num_tiles;
-         tile += (int64_t)gridDim.x * kTableGroups)
+    unsigned char *const group_flag = DESC ? nullptr : flags + grp * kTableBlock * kMergeIPT;
+    const int64_t stride = (int64_t)gridDim.x * kTableGroups;
+    int64_t tile = (int64_t)blockIdx.x * kTableGroups + grp;
+    int32_t sx = 0, ex = 0;
+    if (DESC && tile < num_tiles) {
+        sx = __ldg(coords_x + tile);
+        ex = __ldg(coords_x + tile + 1);
+    }
+    for (; tile < num_tiles; tile += stride) {
+        // DESC: the group's next tile's coordinates, one tile ahead -- every other load of a tile
+        // depends on them
+        int32_t next_sx = 0, next_ex = 0;
+        if (DESC && tile + stride < num_tiles) {
+            next_sx = __ldg(coords_x + tile + stride);
+            next_ex = __ldg(coords_x + tile + stride + 1);
+        }
         merge_tile_reg_body<kTableBlock, HAS_PEERS, true, kTableGroups, OffT, ValT>(
             n_rows, nnz, Ap, Aj, Ax, x, y, alpha_dev, peers, coords_x, carry_row, carry_val, x_hot_biased, tile,
-            groups + grp, table, table_n);
+            groups + grp, table, table_n, group_flag, sx, ex, desc);
+        sx = next_sx;
+        ex = next_ex;
+    }
 }
 #undef MERGE_REG_KERNEL_ARGS
+
+// The tile descriptors (TileDesc) of a partition, one thread per row: the tile in which row r's end
+// item lies is (r + Ap[r+1]) / tile_items (the merge path puts it at diagonal r + Ap[r+1]).  The
+// start mask must be zero on entry.
+template <typename OffT>
+__global__ void __launch_bounds__(256)
+tile_desc_kernel(int32_t n_rows, OffT nnz, const OffT *__restrict__ Ap, const int32_t *__restrict__ coords_x,
+                 uint16_t *__restrict__ row_end, uint32_t *__restrict__ start_mask) {
+    constexpr int SLOTS = kTableBlock * kMergeIPT;
+    constexpr int TILE = SLOTS - 4;
+    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n_rows) return;
+    const int64_t total = (int64_t)n_rows + (int64_t)nnz;
+    const int64_t e = (int64_t)__ldg(Ap + r + 1);
+    const int64_t t = (r + e) / TILE;
+    const int64_t d0 = t * TILE;
+    const int64_t d1 = d0 + TILE < total ? d0 + TILE : total;
+    const int64_t sy = d0 - __ldg(coords_x + t);
+    const int64_t ey = d1 - __ldg(coords_x + t + 1);
+    const int q = (int)(e - sy);
+    row_end[r] = (uint16_t)q;
+    // row r+1 starts inside the tile (q < Z): slot q + shift, as the flag scatter sets it
+    if (e < ey) {
+        const int s = q + (int)(sy & 3);
+        atomicOr(start_mask + t * (SLOTS / 32) + (s >> 5), 1u << (s & 31));
+    }
+}
 
 // ------------------------------------------------------------------------- carry fixup
 // One thread per tile.  Consecutive tiles whose carry lands in the same row form a run; the
@@ -1182,7 +1303,15 @@ int launch_merge(const SpmvProblem<OffT, ValT> &p) {
         const bool tbl_ok = RB == kTableBlock &&
                             (tbl_opt > 0 || (tbl_opt < 0 && sizeof(ValT) == 4 && flags_form &&
                                              num_tiles >= (int64_t)tdi->sm_count * kTableGroups * 4));
-        constexpr int64_t tile_smem = (int64_t)sizeof(TileSmem<kTableBlock, ValT>) * kTableGroups;
+        constexpr bool desc_used = tile_desc_used<kTableGroups, OffT, ValT>();
+        constexpr int64_t flag_smem = (int64_t)kTableGroups * kTableBlock * kMergeIPT;
+        constexpr int64_t tile_smem = (int64_t)sizeof(TileSmem<kTableBlock, ValT>) * kTableGroups +
+                                      (desc_used ? 0 : flag_smem);
+        // What the option charges per tile in flight: its shared memory and its 1 KB of row-start
+        // flags, also where the start mask replaces them, so that the option gives the table sizes
+        // measured below either way.  At the defaults the 8 KB left over do not move the carveout off
+        // its step (100 KB), so the L1 does not gain them either.
+        constexpr int64_t tile_charge = (int64_t)sizeof(TileSmem<kTableBlock, ValT>) * kTableGroups + flag_smem;
         // The option is per SM (every CTA has 1 KB reserved by the system inside a carveout size);
         // -1 = by the size of x.  What the table takes, the L1 loses, in the carveout's steps
         // (100 / 132 / 164 / 196 KB): while x sits in the L2 (R-MAT scale 24) 163 KB is the best size
@@ -1194,7 +1323,7 @@ int launch_merge(const SpmvProblem<OffT, ValT> &p) {
         if (tbl_bytes < 0) tbl_bytes = big_x ? 99 << 10 : 163 << 10;
         if (tbl_bytes > 226 << 10) tbl_bytes = 226 << 10;
         tbl_bytes = (tbl_bytes + 1024) / kTableCtas - 1024;
-        const int64_t k_table = tbl_ok && tbl_bytes > tile_smem ? (tbl_bytes - tile_smem) / (int64_t)sizeof(ValT) : 0;
+        const int64_t k_table = tbl_ok && tbl_bytes > tile_charge ? (tbl_bytes - tile_charge) / (int64_t)sizeof(ValT) : 0;
         const bool want_hot = hot_opt > 0 || (hot_opt < 0 && p.reuse_partition && (big_x || k_table > 0));
         const int64_t k_max = (hot_opt > 0 || big_x) ? option_get("hot_x_max_bytes", 32 << 20) / (int64_t)sizeof(ValT)
                                                      : k_table;
@@ -1217,6 +1346,25 @@ int launch_merge(const SpmvProblem<OffT, ValT> &p) {
                 const int64_t cap = option_get("hot_x_table_limit", -1);   // experiments: fewer entries than planned
                 if (cap >= 0 && cap < tn) tn = cap;
                 const uint32_t table_n = (uint32_t)tn;
+                // the tile descriptors: built once per search of the partition, reused with it
+                void *row_end = nullptr, *start_mask = nullptr;
+                constexpr int64_t mask_bytes = kTableBlock * kMergeIPT / 8;
+                if (desc_used) {
+                    SPMV_TRY(scratch_get(p.stream, SCRATCH_ROW_END, (size_t)p.n_rows * sizeof(uint16_t), &row_end));
+                    SPMV_TRY(scratch_get(p.stream, SCRATCH_START_MASK, (size_t)(num_tiles * mask_bytes), &start_mask));
+                }
+                if (desc_used && !tile_desc_current(p.stream, row_end, start_mask)) {
+                    SPMV_CUDA_TRY(cudaMemsetAsync(start_mask, 0, (size_t)(num_tiles * mask_bytes), p.stream));
+                    if (p.n_rows > 0) {
+                        tile_desc_kernel<OffT><<<(unsigned)(((int64_t)p.n_rows + 255) / 256), 256, 0, p.stream>>>(
+                            p.n_rows, p.nnz, p.Ap, (const int32_t *)coords, static_cast<uint16_t *>(row_end),
+                            static_cast<uint32_t *>(start_mask));
+                        SPMV_LAUNCH_CHECK();
+                    }
+                    tile_desc_store(p.stream, row_end, start_mask);
+                }
+                const TileDesc desc{static_cast<const uint16_t *>(row_end),
+                                    static_cast<const unsigned char *>(start_mask)};
                 const size_t smem = (size_t)tile_smem + (size_t)table_n * sizeof(ValT);
                 SPMV_TRY(apply_max_dynamic_smem(reinterpret_cast<const void *>(tkernel), (int64_t)smem));
                 const DeviceInfo *di = tdi;
@@ -1228,7 +1376,7 @@ int launch_merge(const SpmvProblem<OffT, ValT> &p) {
                 SPMV_CUDA_TRY(cudaLaunchKernelEx(&lc.cfg, tkernel, p.n_rows, p.nnz, p.Ap, hot->Aj2, p.Ax, p.x, p.y,
                                                  p.alpha_dev, p.peers, (const int32_t *)coords,
                                                  static_cast<int32_t *>(crow), static_cast<ValT *>(cval),
-                                                 x_hot_biased, x_hot, table_n, num_tiles));
+                                                 x_hot_biased, x_hot, table_n, num_tiles, desc));
             } else {
             auto kernel = flags_form ? (mc_f32    ? merge_tile_hot_kernel<1, RB, 2, OffT, ValT>
                                         : has_peers ? merge_tile_hot_kernel<1, RB, 1, OffT, ValT>

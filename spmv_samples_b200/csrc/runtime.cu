@@ -31,6 +31,7 @@ struct ScratchBuf {
 struct ScratchSet {
     ScratchBuf slot[SCRATCH_NUM_SLOTS];
     PartitionTag last_partition{nullptr, nullptr, -1, -1, -1, -1};
+    const void *tile_desc[2] = {nullptr, nullptr};  // where the descriptors of last_partition are
 };
 std::map<std::pair<int, cudaStream_t>, ScratchSet> g_scratch;
 
@@ -165,7 +166,24 @@ void partition_tag_store(cudaStream_t stream, const PartitionTag &tag) {
     int dev = -1;
     if (cudaGetDevice(&dev) != cudaSuccess) return;
     std::lock_guard<std::mutex> lk(g_mu);
-    g_scratch[{dev, stream}].last_partition = tag;
+    ScratchSet &set = g_scratch[{dev, stream}];
+    set.last_partition = tag;
+    set.tile_desc[0] = set.tile_desc[1] = nullptr;  // new coordinates: the descriptors are stale
+}
+bool tile_desc_current(cudaStream_t stream, const void *row_end, const void *start_mask) {
+    int dev = -1;
+    if (cudaGetDevice(&dev) != cudaSuccess) return false;
+    std::lock_guard<std::mutex> lk(g_mu);
+    auto it = g_scratch.find({dev, stream});
+    return it != g_scratch.end() && it->second.tile_desc[0] == row_end && it->second.tile_desc[1] == start_mask;
+}
+void tile_desc_store(cudaStream_t stream, const void *row_end, const void *start_mask) {
+    int dev = -1;
+    if (cudaGetDevice(&dev) != cudaSuccess) return;
+    std::lock_guard<std::mutex> lk(g_mu);
+    ScratchSet &set = g_scratch[{dev, stream}];
+    set.tile_desc[0] = row_end;
+    set.tile_desc[1] = start_mask;
 }
 
 void scratch_release_all() {
