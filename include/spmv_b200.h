@@ -116,7 +116,10 @@ SPMVB200_DECLARE_KIND(cusparse)
 /* Generalised SpMV  y[r] = REDUCE_k COMBINE(Ax[k], x[Aj[k]])  from IDENTITY: the fixed menu that
  * stands in for the template functor of the reference's SpMV_merge_based_generalized
  * (merge_genl/merge_genl.cuh:19-38, cpu_navie.hpp:20-35).  Served by the merge-path kernel only
- * (kind merge or auto), as in the reference.  Empty rows yield IDENTITY. */
+ * (kind merge or auto), as in the reference.  Empty rows yield IDENTITY.
+ * Min-plus and max-plus with infinite x (an unreached vertex is x = +inf) follow IEEE; when a
+ * combine yields NaN (+inf + -inf, or a NaN input) the result is unspecified: it depends on where
+ * the NaN meets the reduction (min(u, v) as u < v ? u : v forgets a NaN once a later term comes). */
 enum {
     SPMVB200_SEMIRING_PLUS_TIMES = 0, /* 0,    a*x,            u+v        (ordinary SpMV)     */
     SPMVB200_SEMIRING_MIN_PLUS = 1,   /* +inf, a+x,            min(u,v)   (shortest paths)    */
@@ -130,7 +133,12 @@ enum {
  * still holds what it held at the previous call on this stream, so the merge-path kernel may
  * reuse that call's tile coordinates instead of searching again (an iterative solver's matrix;
  * the reference re-derives everything per call, merge_based/dispatch_spmv_orig.cuh:613-660).
- * The first call on a matrix, or any call after Ap's contents changed, must not pass it. */
+ * The first call on a matrix, or any call after Ap's contents changed, must not pass it.
+ * Special values (every kind, SpMM and the beta form): Inf and NaN propagate per IEEE within their
+ * own row only -- a row is NaN if one of its products is NaN or it has both a +inf and a -inf
+ * product, else +-inf if it has a product of that sign -- and never reach another row.  Stored
+ * zeros are multiplied, as cuSPARSE does: 0 * inf in a row makes it NaN.  Subnormal values are
+ * kept (the library is not built to flush them to zero). */
 #define SPMVB200_FLAG_STATIC_PATTERN 1
 typedef struct {
     int32_t kind;

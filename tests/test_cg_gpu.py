@@ -163,6 +163,30 @@ def test_cg_breakdown_on_negative_definite(jacobi):
     assert bool(torch.isfinite(res.x).all())
 
 
+@pytest.mark.parametrize("jacobi", [False, True])
+@pytest.mark.parametrize("poison", ["nan_in_b", "inf_in_x0", "nan_off_diagonal"])
+@pytest.mark.parametrize("dtype", [np.float32, np.float64], ids=["f32", "f64"])
+def test_cg_non_finite_input_breaks_down_at_once(dtype, poison, jacobi):
+    """A NaN or an inf present from the start makes r.z (or ||b||) non-finite in the set-up: the
+    solve reports a breakdown before the first iteration instead of iterating on NaN."""
+    from spmv_samples_b200 import solve
+    Ap, Aj, Ax, b, (dAp, dAj, dAx, db) = problem(32, dtype)
+    n = Ap.shape[0] - 1
+    x0 = torch.zeros_like(db)
+    if poison == "nan_in_b":
+        db = db.clone()
+        db[n // 2] = float("nan")
+    elif poison == "inf_in_x0":
+        x0[n // 3] = float("inf")
+    else:
+        rows = np.repeat(np.arange(n), np.diff(Ap))
+        k = int(np.nonzero(Aj != rows)[0][len(Aj) // 3])
+        dAx = dAx.clone()
+        dAx[k] = float("nan")
+    res = solve.cg(dAp, dAj, dAx, db, x0, rtol=1e-6, jacobi=jacobi)
+    assert res.breakdown and not res.converged and res.iterations == 0, res
+
+
 def test_cg_jacobi_rejects_a_bad_diagonal():
     from spmv_samples_b200 import _lib, solve
     Ap, Aj, Ax, b, _ = problem(16)

@@ -342,11 +342,15 @@ def cuda(built_lib):
 class Case:
     """One exact test case on the device: pattern, integer values, int64 expectation."""
 
-    def __init__(self, name, lens, off, val, seed, spare_bits=0):
+    def __init__(self, name, lens, off, val, seed, spare_bits=0, x_exp=0):
         self.name = name
         self.Ap, self.Aj = pattern(lens, seed, off=off)
-        self.Ax, self.x, _, _ = exact_inputs(self.Ap, self.Aj, N_COLS, val, seed, spare_bits)
-        self.y_ref = exact_reference(self.Ap, self.Aj, self.Ax, self.x)
+        self.Ax, x, _, _ = exact_inputs(self.Ap, self.Aj, N_COLS, val, seed, spare_bits)
+        self.y_ref = exact_reference(self.Ap, self.Aj, self.Ax, x)
+        # x scaled by 2^x_exp: products and partial sums stay exact, y is y_ref * 2^x_exp
+        self.x_scale = 2.0 ** x_exp
+        self.x = np.ldexp(x, x_exp).astype(x.dtype)
+        assert np.all(self.x.astype(np.float64) == x.astype(np.float64) * self.x_scale)
         self.n_rows = self.Ap.size - 1
         self.d = [torch.from_numpy(np.ascontiguousarray(a)).cuda() for a in (self.Ap, self.Aj, self.Ax, self.x)]
 
@@ -356,7 +360,7 @@ class Case:
     def check(self, y, what, scale=1.0, y0=None):
         """y == scale * (A x) [+ beta-term y0], compared exactly (all values are exact in fp64)."""
         got = y.cpu().numpy().astype(np.float64)
-        want = self.y_ref.astype(np.float64) * scale
+        want = self.y_ref.astype(np.float64) * (scale * self.x_scale)
         if y0 is not None:
             want = want + y0
         bad = np.nonzero(got != want)[0]
@@ -364,8 +368,8 @@ class Case:
                                f"{bad[:5].tolist()}: got {got[bad[:5]].tolist()}, want {want[bad[:5]].tolist()}")
 
 
-def cases(shapes, off, val, spare_bits=0):
-    return [Case(n, lens, off, val, i, spare_bits) for i, (n, lens) in enumerate(sorted(shapes.items()))]
+def cases(shapes, off, val, spare_bits=0, x_exp=0):
+    return [Case(n, lens, off, val, i, spare_bits, x_exp) for i, (n, lens) in enumerate(sorted(shapes.items()))]
 
 
 def run(kind, c, **kw):
@@ -595,6 +599,57 @@ def test_spmm_exact(cuda, off, val, route, k):
                 assert bool(torch.isnan(Yb[:, k:]).all()), "SpMM wrote past k in a row of Y"
 
 
+# ---------------------------------------------------------------------------------- range edges
+# x scaled by a power of two: subnormal (every x and many y below the smallest normal number; fp32
+# x are multiples of 2^-140 >= 2^-149, fp64 x of 2^-1060 >= 2^-1074, so all stay exact) and the top
+# of the range (|y| < 2^24 * 2^100 < 2^128 in fp32, < 2^53 * 2^900 in fp64).  A build that flushes
+# subnormals to zero, or an intermediate held in a narrower type, changes y.
+X_EXP = {"subnormal": {np.float32: -140, np.float64: -1060}, "top": {np.float32: 100, np.float64: 900}}
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("kind", ["merge", "merge_table", "vector", "light", "stream", "spmm"])
+@pytest.mark.parametrize("where", sorted(X_EXP))
+@pytest.mark.parametrize("off,val", OFF_VAL, ids=OV_IDS)
+def test_subnormal_and_top_of_range_exact(cuda, off, val, where, kind):
+    from spmv_samples_b200 import spmv
+    e = X_EXP[where][val]
+    reg, _ = merge_tiles()
+    if kind in ("merge", "merge_table"):
+        shapes = all_merge_shapes()
+    elif kind == "spmm":
+        shapes = merge_shapes(508)
+    else:
+        shapes = {**{"vector": vector_shapes(), "light": light_shapes(), "stream": stream_shapes()}[kind],
+                  **{k: v for k, v in merge_shapes(reg).items() if "mod8" in k}}
+    cs = cases(shapes, off, val, x_exp=e)
+    tiny = np.finfo(val).tiny
+    if where == "subnormal":
+        assert all(np.all(np.abs(c.x) < tiny) for c in cs)
+        assert sum(int(np.count_nonzero((c.y_ref != 0) & (np.abs(c.y_ref * c.x_scale) < tiny))) for c in cs) > 0
+    opts = _merge_opts("table", 1, np.dtype(val).itemsize) if kind == "merge_table" else {}
+    try:
+        with options(**opts):
+            for c in cs:
+                if kind != "spmm":
+                    spmv.release_cache()
+                    c.check(run(kind.split("_")[0], c), f"{kind} x * 2^{e}")
+                    continue
+                # k = 4 columns: x * 2^e and three more exact vectors at the same scale
+                tdt = torch.float32 if val == np.float32 else torch.float64
+                xs = [c.x] + [np.ldexp(exact_inputs(c.Ap, c.Aj, N_COLS, val, 100 + j)[1], e).astype(val)
+                              for j in range(1, 4)]
+                X = torch.from_numpy(np.stack(xs, axis=1)).cuda()
+                Y = torch.full((c.n_rows, 4), float("nan"), dtype=tdt, device="cuda")
+                spmv.spmm(c.d[0], c.d[1], c.d[2], X, Y)
+                torch.cuda.synchronize()
+                for j in range(4):
+                    want = exact_reference(c.Ap, c.Aj, c.Ax, np.ldexp(xs[j], -e)).astype(np.float64) * c.x_scale
+                    assert np.array_equal(Y[:, j].cpu().numpy().astype(np.float64), want), (c.name, j)
+    finally:
+        spmv.release_cache()
+
+
 # ---------------------------------------------------------------------------------- generalised kernel
 @pytest.mark.gpu
 @pytest.mark.parametrize("off,val", OFF_VAL, ids=OV_IDS)
@@ -616,6 +671,11 @@ def test_generalised_kernel_exact_on_its_tile_edges(cuda, off, val):
         spmv.spmv_ex("merge", *c.d, y, n_cols=N_COLS, beta_dev=beta)
         torch.cuda.synchronize()
         c.check(y, "A x + beta y", y0=-2.0 * y0.astype(np.float64))
+        # beta = 0: y is not read (BLAS), so a NaN there does not reach the result
+        y = c.y(float("nan"))
+        spmv.spmv_ex("merge", *c.d, y, n_cols=N_COLS, beta_dev=torch.zeros(1, dtype=tdt, device="cuda"))
+        torch.cuda.synchronize()
+        c.check(y, "A x + 0 * NaN")
         x = c.x.copy()
         x[::7] = 0                                          # or-and sees zeros
         dx = torch.from_numpy(x).cuda()
