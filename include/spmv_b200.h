@@ -225,6 +225,25 @@ typedef struct {
 } spmvb200_cg_result_t;
 SPMVB200_API int spmvb200_cg(const spmvb200_cg_args_t *args, spmvb200_cg_result_t *out);
 
+/* ---- BiCGSTAB solve A x = b on the device (csrc/bicgstab.cu) -------------------------------
+ * A is n x n in CSR and need not be symmetric; right-preconditioned BiCGSTAB (van der Vorst) with
+ * M = I, or M = diag(A) with SPMVB200_CG_JACOBI, in the operation order of
+ * scipy.sparse.linalg.bicgstab.  Takes the records of spmvb200_cg (spmvb200_cg_args_t,
+ * spmvb200_cg_result_t) with the same meaning, the same argument checks and status codes; n == 0
+ * reports convergence after 0 iterations.  One iteration is two SpMVs of `kind`
+ * (SPMVB200_FLAG_STATIC_PATTERN on every call after the first) and five streaming kernels; dot
+ * products accumulate in double in a fixed order, so a solve is deterministic for the
+ * deterministic kinds.  `iterations` counts the times x was moved along the search direction, so
+ * a solve that converges at the half step (||s|| <= rtol * ||b||) counts that iteration.  It stops
+ * when the recursive residual meets ||r|| <= rtol * ||b|| (or ||s|| does), after max_iter
+ * iterations, or at a breakdown: an exact zero or a non-finite value of (r^, r), (r^, v), alpha,
+ * (t, t) or omega, or omega == 0 -- the method cannot continue (e.g. (r^, v) = 0 for the shadow
+ * residual r^ = r0), or the input holds NaN or inf.  A breakdown is not an error; x is then the
+ * last finite iterate.  residual_norm is ||b - A x|| of the returned x, computed once more in
+ * fp64.  Workspace (5 vectors, 8 with Jacobi) is cached per (device, stream) and freed by
+ * spmvb200_release_cache. */
+SPMVB200_API int spmvb200_bicgstab(const spmvb200_cg_args_t *args, spmvb200_cg_result_t *out);
+
 /* ---- merge-path partition, exposed so parity tests can demand bit-exact coordinates --- */
 /* Row coordinate of the merge path on each diagonal min(t * tile_items, n_rows + nnz),
  * t = 0 .. n_coords-1, written to the DEVICE array coords_x (int32).  The nonzero

@@ -23,6 +23,8 @@
 //   --cg RTOL [--jacobi]: for a square matrix, b = A*1 and x0 = 0, then one conjugate-gradient solve
 //   (Jacobi-preconditioned with --jacobi) per kind through spmvb200_cg; exits non-zero if one does
 //   not converge
+//   --bicgstab RTOL [--jacobi]: the same with one BiCGSTAB solve per kind (spmvb200_bicgstab), for a
+//   square matrix that need not be symmetric
 #include <algorithm>
 #include <chrono>
 #include <cmath>
@@ -59,7 +61,8 @@ struct Options {
     int gpus = 1;    // --gpus N: the row-sharded power iteration over N GPUs of this box
     int power = 0;   // --power K: K power-iteration steps x <- A x / ||A x|| (BASELINE.json configs[4])
     double cg_rtol = 0;      // --cg RTOL: one CG solve of A x = A*1 per kind
-    bool cg_jacobi = false;  // --jacobi: with M = diag(A)
+    double bicgstab_rtol = 0;  // --bicgstab RTOL: one BiCGSTAB solve of A x = A*1 per kind
+    bool cg_jacobi = false;  // --jacobi: with M = diag(A) (both solvers)
 };
 
 template <typename T>
@@ -80,9 +83,13 @@ static int kind_id(const string &k) {
     return -1;
 }
 
-// --cg: b = A*1, x0 = 0, one solve per kind; returns the number of kinds that did not converge
+using KrylovSolve = int (*)(const spmvb200_cg_args_t *, spmvb200_cg_result_t *);
+
+// --cg / --bicgstab: b = A*1, x0 = 0, one solve per kind by `solve` (spmvb200_cg or
+// spmvb200_bicgstab); returns the number of kinds that did not converge
 template <typename offset_t, typename value_t>
-static int run_cg(const Options &opt, index_t n, offset_t nnz, offset_t *dAp, index_t *dAj, value_t *dAx) {
+static int run_krylov(const Options &opt, KrylovSolve solve, const char *title, double rtol, index_t n, offset_t nnz,
+                      offset_t *dAp, index_t *dAj, value_t *dAx) {
     const size_t vb = sizeof(value_t);
     vector<value_t> ones((size_t)n, value_t(1)), hx((size_t)n);
     value_t *d1 = device_alloc<value_t>((size_t)n), *dB = device_alloc<value_t>((size_t)n);
@@ -105,7 +112,7 @@ static int run_cg(const Options &opt, index_t n, offset_t nnz, offset_t *dAp, in
     cudaEvent_t e0, e1;
     checkCudaErr(cudaEventCreate(&e0));
     checkCudaErr(cudaEventCreate(&e1));
-    printf("Conjugate gradients (b = A*1, x0 = 0, rtol %.1e%s, max %d iterations):\n", opt.cg_rtol,
+    printf("%s (b = A*1, x0 = 0, rtol %.1e%s, max %d iterations):\n", title, rtol,
            opt.cg_jacobi ? ", Jacobi preconditioner" : "", n);
     int failures = 0;
     for (const auto &kind : opt.kinds) {
@@ -129,11 +136,11 @@ static int run_cg(const Options &opt, index_t n, offset_t nnz, offset_t *dAp, in
         a.Ax = dAx;
         a.b = dB;
         a.x = dX;
-        a.rtol = opt.cg_rtol;
+        a.rtol = rtol;
         a.max_iter = n;
         spmvb200_cg_result_t r;
         checkCudaErr(cudaEventRecord(e0, nullptr));
-        checkSpmvStatus(spmvb200_cg(&a, &r));  // synchronises
+        checkSpmvStatus(solve(&a, &r));  // synchronises
         checkCudaErr(cudaEventRecord(e1, nullptr));
         checkCudaErr(cudaEventSynchronize(e1));
         float ms = 0.f;
@@ -291,11 +298,18 @@ static int run(const Options &opt, const string &name, index_t n_rows, index_t n
         spmvb200_power_destroy(pw);
     }
 
-    if (opt.cg_rtol > 0) {
+    const struct {
+        double rtol;
+        KrylovSolve solve;
+        const char *title;
+    } solves[] = {{opt.cg_rtol, spmvb200_cg, "Conjugate gradients"}, {opt.bicgstab_rtol, spmvb200_bicgstab, "BiCGSTAB"}};
+    for (const auto &sv : solves) {
+        if (sv.rtol <= 0) continue;
         if (n_rows == n_cols) {
-            failures += run_cg<offset_t, value_t>(opt, n_rows, nnz, dA_csrOffsets, dA_columns, dA_values);
+            failures += run_krylov<offset_t, value_t>(opt, sv.solve, sv.title, sv.rtol, n_rows, nnz, dA_csrOffsets,
+                                                      dA_columns, dA_values);
         } else {
-            printf("Conjugate gradients: the matrix is not square\n");
+            printf("%s: the matrix is not square\n", sv.title);
             ++failures;
         }
     }
@@ -390,7 +404,7 @@ static int run_synthetic(const Options &opt, const string &cfg, long size) {
 int main(int argc, char **argv) {
     if (argc < 3) {
         cerr << "usage: ./bin/<program-name>  <filename.mtx | synthetic:c1..c5[:size]>  <SpMV_kind_string>..."
-                "  [--iters N] [--x ones|random] [--flush] [--dynamic-pattern] [--peak GB/s] [--power K [--gpus N]] [--cg RTOL [--jacobi]]"
+                "  [--iters N] [--x ones|random] [--flush] [--dynamic-pattern] [--peak GB/s] [--power K [--gpus N]] [--cg RTOL] [--bicgstab RTOL] [--jacobi]"
              << endl;
         exit(1);
     }
@@ -406,6 +420,7 @@ int main(int argc, char **argv) {
         else if (a == "--gpus" && i + 1 < argc) opt.gpus = atoi(argv[++i]);
         else if (a == "--power" && i + 1 < argc) opt.power = atoi(argv[++i]);
         else if (a == "--cg" && i + 1 < argc) opt.cg_rtol = atof(argv[++i]);
+        else if (a == "--bicgstab" && i + 1 < argc) opt.bicgstab_rtol = atof(argv[++i]);
         else if (a == "--jacobi") opt.cg_jacobi = true;
         else opt.kinds.push_back(a);
     }

@@ -8,7 +8,8 @@ Python package is the thin binding used by tests, bench.py and the multi-GPU dri
     spmv      SpMV(kind_str, n_rows, n_cols, nnz, Ap, Aj, Ax, x, y) and SPMV_KINDS
     generate  device-side synthetic matrices (BASELINE.json configs c1..c5)
     matrix    CsrMatrix: host-buffer (end-to-end) front end
-    solve     cg(): conjugate-gradient solve on the device, optionally Jacobi-preconditioned
+    solve     cg(): conjugate-gradient solve on the device (SPD matrices), bicgstab(): BiCGSTAB
+              for general square matrices; both optionally Jacobi-preconditioned
 
 Importing the package does not need a GPU; calling into it does, and nothing falls back.
 """

@@ -105,6 +105,8 @@ def lib() -> C.CDLL:
     L.spmvb200_spmm.restype = C.c_int
     L.spmvb200_cg.argtypes = [C.POINTER(CgArgs), C.POINTER(CgOut)]
     L.spmvb200_cg.restype = C.c_int
+    L.spmvb200_bicgstab.argtypes = [C.POINTER(CgArgs), C.POINTER(CgOut)]
+    L.spmvb200_bicgstab.restype = C.c_int
     L.spmvb200_launch_count.restype = C.c_int64
     L.spmvb200_get_option.restype = C.c_int64
     L.spmvb200_get_option.argtypes = [C.c_char_p]

@@ -7,25 +7,19 @@
 //   cg_update_kernel     x += alpha p, r -= alpha q, z = dinv r (Jacobi); r.z, r.r
 //                                                     -> beta = rho' / rho, converged, iteration += 1
 //   cg_direction_kernel  p = z + beta p
-// Every dot product accumulates in double in a fixed order: per-block partials, then the last
-// block to finish (threadfence + counter, as norm_exchange_kernel in power.cu) adds them in block
-// order.  The scalars live in a small device state block, so the host never reads them inside the
-// loop: it enqueues iterations in batches of 1, 2, 4, ... kCgMaxBatch and reads the flags once per
-// batch.  Every CG kernel returns at once when `converged` or `breakdown` is set, so x and the
+// Every dot product accumulates in double in a fixed order (grid_sum, krylov.cuh).  The scalars
+// live in a small device state block, so the host never reads them inside the loop: it enqueues
+// iterations in batches of 1, 2, 4, ... kKrylovMaxBatch and reads the flags once per batch.  Every CG kernel returns at once when `converged` or `breakdown` is set, so x and the
 // iteration count are those of the iteration where the criterion first held, whatever the batch
 // boundaries (the SpMVs left in a batch still run; they only rewrite q).
 #include <algorithm>
 #include <cmath>
 #include <cstring>
 
-#include "common.cuh"
+#include "krylov.cuh"
 
 namespace spmvb200 {
 namespace {
-
-constexpr int kCgBlock = 256;
-constexpr int kCgBlocksPerSm = 8;
-constexpr int64_t kCgMaxBatch = 64;  // iterations enqueued between two reads of the flags, at most
 
 struct CgState {
     double rho;    // r.z of the current residual
@@ -44,80 +38,9 @@ struct CgState {
 
 __device__ __forceinline__ bool cg_stopped(const CgState *st) { return (st->converged | st->breakdown) != 0; }
 
-// N block sums in a fixed order; the totals are valid in thread 0
-template <int N>
-__device__ __forceinline__ void block_sum(double (&v)[N]) {
-    __shared__ double s[N][kCgBlock / 32];
-#pragma unroll
-    for (int j = 0; j < N; ++j) {
-#pragma unroll
-        for (int d = 16; d > 0; d >>= 1) v[j] += __shfl_xor_sync(0xffffffffu, v[j], d);
-        if ((threadIdx.x & 31) == 0) s[j][threadIdx.x >> 5] = v[j];
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-#pragma unroll
-        for (int j = 0; j < N; ++j) {
-            double t = 0.0;
-#pragma unroll
-            for (int w = 0; w < kCgBlock / 32; ++w) t += s[j][w];
-            v[j] = t;
-        }
-    }
-    __syncthreads();  // s may be reused
-}
-
-// Grid-wide sums of v: true in the last block to finish, whose thread 0 then holds the totals,
-// added in block order (the same bits on every run with the same grid).
-template <int N>
-__device__ __forceinline__ bool grid_sum(double (&v)[N], double *partial, unsigned int *counter) {
-    __shared__ bool is_last;
-    block_sum<N>(v);
-    if (threadIdx.x == 0) {
-#pragma unroll
-        for (int j = 0; j < N; ++j) partial[(size_t)j * gridDim.x + blockIdx.x] = v[j];
-        __threadfence();
-        is_last = atomicAdd(counter, 1u) == gridDim.x - 1;
-    }
-    __syncthreads();
-    if (!is_last) return false;
-    __threadfence();
-#pragma unroll
-    for (int j = 0; j < N; ++j) {
-        v[j] = 0.0;
-        for (int i = threadIdx.x; i < (int)gridDim.x; i += kCgBlock) v[j] += __ldcg(partial + (size_t)j * gridDim.x + i);
-    }
-    block_sum<N>(v);
-    if (threadIdx.x == 0) *counter = 0;  // ready for the next reduction
-    return true;
-}
-
-__device__ __forceinline__ int64_t first_index() { return (int64_t)blockIdx.x * kCgBlock + threadIdx.x; }
-__device__ __forceinline__ int64_t grid_stride() { return (int64_t)gridDim.x * kCgBlock; }
-
-// dinv[i] = 1 / A[i,i]: row i searched for column i (duplicates are added, as the SpMV adds them)
-template <typename OffT, typename ValT>
-__global__ void __launch_bounds__(kCgBlock)
-jacobi_diag_kernel(int64_t n, const OffT *__restrict__ Ap, const int32_t *__restrict__ Aj,
-                   const ValT *__restrict__ Ax, ValT *__restrict__ dinv, CgState *st) {
-    for (int64_t i = first_index(); i < n; i += grid_stride()) {
-        double d = 0.0;
-        bool found = false;
-        for (OffT k = Ap[i]; k < Ap[i + 1]; ++k) {
-            if (Aj[k] == (int32_t)i) {
-                d += (double)Ax[k];
-                found = true;
-            }
-        }
-        const bool ok = found && d != 0.0;
-        if (!ok) st->bad_diag = 1;
-        dinv[i] = ok ? (ValT)(1.0 / d) : ValT(0);
-    }
-}
-
 // r = b - q (q = A x0), z = dinv r, p = z; rho = r.z, ||r||^2, ||b||^2
 template <typename ValT, bool kJacobi>
-__global__ void __launch_bounds__(kCgBlock)
+__global__ void __launch_bounds__(kKrylovBlock)
 cg_init_kernel(int64_t n, const ValT *__restrict__ b, const ValT *__restrict__ q, const ValT *__restrict__ dinv,
                ValT *__restrict__ r, ValT *__restrict__ z, ValT *__restrict__ p, double rtol, CgState *st,
                double *__restrict__ partial) {
@@ -150,7 +73,7 @@ cg_init_kernel(int64_t n, const ValT *__restrict__ b, const ValT *__restrict__ q
 
 // p.q -> alpha
 template <typename ValT>
-__global__ void __launch_bounds__(kCgBlock)
+__global__ void __launch_bounds__(kKrylovBlock)
 cg_pq_kernel(int64_t n, const ValT *__restrict__ p, const ValT *__restrict__ q, CgState *st,
              double *__restrict__ partial) {
     if (cg_stopped(st)) return;
@@ -166,7 +89,7 @@ cg_pq_kernel(int64_t n, const ValT *__restrict__ p, const ValT *__restrict__ q, 
 
 // x += alpha p, r -= alpha q, z = dinv r; r.z and r.r -> converged / beta, one more iteration
 template <typename ValT, bool kJacobi>
-__global__ void __launch_bounds__(kCgBlock)
+__global__ void __launch_bounds__(kKrylovBlock)
 cg_update_kernel(int64_t n, const ValT *__restrict__ p, const ValT *__restrict__ q, const ValT *__restrict__ dinv,
                  ValT *__restrict__ x, ValT *__restrict__ r, ValT *__restrict__ z, CgState *st,
                  double *__restrict__ partial) {
@@ -205,55 +128,11 @@ cg_update_kernel(int64_t n, const ValT *__restrict__ p, const ValT *__restrict__
 
 // p = z + beta p  (z = r without a preconditioner)
 template <typename ValT>
-__global__ void __launch_bounds__(kCgBlock)
+__global__ void __launch_bounds__(kKrylovBlock)
 cg_direction_kernel(int64_t n, const ValT *__restrict__ z, ValT *__restrict__ p, const CgState *st) {
     if (cg_stopped(st)) return;
     const ValT bt = (ValT)st->beta;
     for (int64_t i = first_index(); i < n; i += grid_stride()) p[i] = z[i] + bt * p[i];
-}
-
-// ||b - A x||^2 in fp64, one row per thread: products and sums in double, in row order, without
-// contraction -- per row the same operations as the fp64 host reference, for both value types
-template <typename OffT, typename ValT>
-__global__ void __launch_bounds__(kCgBlock)
-cg_residual_kernel(int64_t n, const OffT *__restrict__ Ap, const int32_t *__restrict__ Aj,
-                   const ValT *__restrict__ Ax, const ValT *__restrict__ x, const ValT *__restrict__ b,
-                   CgState *st, double *__restrict__ partial) {
-    double acc[1] = {0.0};
-    for (int64_t i = first_index(); i < n; i += grid_stride()) {
-        double y = 0.0;
-        for (OffT k = Ap[i]; k < Ap[i + 1]; ++k) y = __dadd_rn(y, __dmul_rn((double)Ax[k], (double)x[Aj[k]]));
-        const double ri = __dsub_rn((double)b[i], y);
-        acc[0] += ri * ri;
-    }
-    if (!grid_sum<1>(acc, partial, &st->counter)) return;
-    if (threadIdx.x == 0) st->res2 = acc[0];
-}
-
-inline size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
-
-int cg_spmv(const spmvb200_cg_args_t &a, const void *in, void *out, int flags) {
-    spmvb200_args_t s;
-    std::memset(&s, 0, sizeof(s));
-    s.kind = a.kind;
-    s.offset_bits = a.offset_bits;
-    s.value_bits = a.value_bits;
-    s.n_rows = s.n_cols = a.n;
-    s.nnz = a.nnz;
-    s.Ap = a.Ap;
-    s.Aj = a.Aj;
-    s.Ax = a.Ax;
-    s.x = in;
-    s.y = out;
-    s.stream = a.stream;
-    s.flags = flags;
-    return spmvb200_spmv(&s);
-}
-
-int read_state(const CgState *st_dev, CgState *h, cudaStream_t stream) {
-    SPMV_CUDA_TRY(cudaMemcpyAsync(h, st_dev, sizeof(CgState), cudaMemcpyDeviceToHost, stream));
-    SPMV_CUDA_TRY(cudaStreamSynchronize(stream));
-    return SPMVB200_OK;
 }
 
 template <typename OffT, typename ValT, bool kJacobi>
@@ -265,10 +144,8 @@ int cg_run(const spmvb200_cg_args_t &a, spmvb200_cg_result_t *out) {
     const ValT *b = static_cast<const ValT *>(a.b);
     ValT *x = static_cast<ValT *>(a.x);
 
-    const DeviceInfo *di = nullptr;
-    SPMV_TRY(current_device_info(&di));
-    const int64_t cap = (int64_t)di->sm_count * kCgBlocksPerSm;
-    const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + kCgBlock - 1) / kCgBlock, cap));
+    unsigned grid = 0;
+    SPMV_TRY(krylov_grid(n, &grid));
 
     // workspace: state | partials (3 sums per block) | r p q [z dinv]
     const size_t off_part = align256(sizeof(CgState));
@@ -287,12 +164,12 @@ int cg_run(const spmvb200_cg_args_t &a, spmvb200_cg_result_t *out) {
 
     SPMV_CUDA_TRY(cudaMemsetAsync(st, 0, sizeof(CgState), s));
     if (kJacobi) {
-        jacobi_diag_kernel<OffT, ValT><<<grid, kCgBlock, 0, s>>>(n, Ap, a.Aj, Ax, dinv, st);
+        jacobi_diag_kernel<OffT, ValT><<<grid, kKrylovBlock, 0, s>>>(n, Ap, a.Aj, Ax, dinv, &st->bad_diag);
         SPMV_LAUNCH_CHECK();
     }
     // r0 = b - A x0: the first SpMV on this matrix, so without the static-pattern flag
-    SPMV_TRY(cg_spmv(a, x, q, 0));
-    cg_init_kernel<ValT, kJacobi><<<grid, kCgBlock, 0, s>>>(n, b, q, dinv, r, z, p, a.rtol, st, partial);
+    SPMV_TRY(krylov_spmv(a, x, q, 0));
+    cg_init_kernel<ValT, kJacobi><<<grid, kKrylovBlock, 0, s>>>(n, b, q, dinv, r, z, p, a.rtol, st, partial);
     SPMV_LAUNCH_CHECK();
     CgState h;
     SPMV_TRY(read_state(st, &h, s));
@@ -302,21 +179,22 @@ int cg_run(const spmvb200_cg_args_t &a, spmvb200_cg_result_t *out) {
     while (!h.converged && !h.breakdown && enqueued < a.max_iter) {
         const int64_t k = std::min(batch, a.max_iter - enqueued);
         for (int64_t it = 0; it < k; ++it) {
-            SPMV_TRY(cg_spmv(a, p, q, SPMVB200_FLAG_STATIC_PATTERN));
-            cg_pq_kernel<ValT><<<grid, kCgBlock, 0, s>>>(n, p, q, st, partial);
+            SPMV_TRY(krylov_spmv(a, p, q, SPMVB200_FLAG_STATIC_PATTERN));
+            cg_pq_kernel<ValT><<<grid, kKrylovBlock, 0, s>>>(n, p, q, st, partial);
             SPMV_LAUNCH_CHECK();
-            cg_update_kernel<ValT, kJacobi><<<grid, kCgBlock, 0, s>>>(n, p, q, dinv, x, r, z, st, partial);
+            cg_update_kernel<ValT, kJacobi><<<grid, kKrylovBlock, 0, s>>>(n, p, q, dinv, x, r, z, st, partial);
             SPMV_LAUNCH_CHECK();
-            cg_direction_kernel<ValT><<<grid, kCgBlock, 0, s>>>(n, z, p, st);
+            cg_direction_kernel<ValT><<<grid, kKrylovBlock, 0, s>>>(n, z, p, st);
             SPMV_LAUNCH_CHECK();
         }
         enqueued += k;
-        batch = std::min(2 * batch, kCgMaxBatch);
+        batch = std::min(2 * batch, kKrylovMaxBatch);
         SPMV_TRY(read_state(st, &h, s));
     }
     // b = 0: the solution is x = 0, whatever x0 was
     if (h.bb == 0.0) SPMV_CUDA_TRY(cudaMemsetAsync(x, 0, (size_t)n * sizeof(ValT), s));
-    cg_residual_kernel<OffT, ValT><<<grid, kCgBlock, 0, s>>>(n, Ap, a.Aj, Ax, x, b, st, partial);
+    krylov_residual_kernel<OffT, ValT><<<grid, kKrylovBlock, 0, s>>>(n, Ap, a.Aj, Ax, x, b, &st->res2, partial,
+                                                                    &st->counter);
     SPMV_LAUNCH_CHECK();
     SPMV_TRY(read_state(st, &h, s));
 

@@ -1,11 +1,13 @@
-"""Conjugate-gradient solve of A x = b on the device (spmvb200_cg, csrc/cg.cu).
+"""Krylov solves of A x = b on the device: conjugate gradients (spmvb200_cg, csrc/cg.cu) for a
+symmetric positive definite A, BiCGSTAB (spmvb200_bicgstab, csrc/bicgstab.cu) for any square A.
 
     res = cg(Ap, Aj, Ax, b, rtol=1e-8, kind="auto", jacobi=True)
+    res = bicgstab(Ap, Aj, Ax, b, rtol=1e-8, kind="auto", jacobi=True)
 
-A is a symmetric positive definite n x n CSR matrix (CUDA tensors, as for spmv.SpMV).  Each
-iteration is one SpMV of the chosen kind and three streaming kernels; the dot products accumulate
-in double in a fixed order, and the host reads the convergence flags once per batch of
-iterations instead of once per iteration.  There is no PyTorch or CPU fallback.
+A is an n x n CSR matrix (CUDA tensors, as for spmv.SpMV).  A CG iteration is one SpMV of the
+chosen kind and three streaming kernels, a BiCGSTAB iteration two SpMVs and five; the dot
+products accumulate in double in a fixed order, and the host reads the convergence flags once
+per batch of iterations instead of once per iteration.  There is no PyTorch or CPU fallback.
 """
 from __future__ import annotations
 
@@ -25,7 +27,7 @@ class CgResult:
     residual_norm: float   # ||b - A x|| of the returned x, computed in fp64
     b_norm: float
     converged: bool        # ||r|| <= rtol * ||b|| for the recursive residual r
-    breakdown: bool        # p.q <= 0 or not finite: A is not SPD (not an error)
+    breakdown: bool        # the method cannot continue (not an error): see cg() and bicgstab()
 
 
 def cg(Ap, Aj, Ax, b, x=None, *, rtol=1e-6, max_iter=None, kind="auto", jacobi=False,
@@ -35,6 +37,23 @@ def cg(Ap, Aj, Ax, b, x=None, *, rtol=1e-6, max_iter=None, kind="auto", jacobi=F
     n.  Stops at the first iteration with ||r|| <= rtol * ||b||, after max_iter iterations, or at a
     breakdown.  Raises SpmvB200Error (status 1) when jacobi=True and a diagonal entry is missing or
     zero."""
+    return _solve("spmvb200_cg", Ap, Aj, Ax, b, x, rtol, max_iter, kind, jacobi, stream)
+
+
+def bicgstab(Ap, Aj, Ax, b, x=None, *, rtol=1e-6, max_iter=None, kind="auto", jacobi=False,
+             stream=None) -> CgResult:
+    """Solve A x = b for a general square A by right-preconditioned BiCGSTAB, with M = diag(A)
+    when jacobi=True, in the operation order of scipy.sparse.linalg.bicgstab.  x: initial guess,
+    overwritten with the solution; None starts from zero.  max_iter: None means n.  Stops when
+    ||r|| <= rtol * ||b|| (also at the half step, ||s|| <= rtol * ||b||, which counts as an
+    iteration), after max_iter iterations, or at a breakdown: an exact zero or a non-finite value
+    of one of the method's scalars, which leaves x at its last finite iterate.  Raises
+    SpmvB200Error (status 1) when jacobi=True and a diagonal entry is missing or zero."""
+    return _solve("spmvb200_bicgstab", Ap, Aj, Ax, b, x, rtol, max_iter, kind, jacobi, stream)
+
+
+def _solve(entry, Ap, Aj, Ax, b, x, rtol, max_iter, kind, jacobi, stream) -> CgResult:
+    """Both solvers: the argument checks, made before touching a device, then the call."""
     for name, t in (("Ap", Ap), ("Aj", Aj), ("Ax", Ax), ("b", b), ("x", x)):
         if t is not None and t.dim() != 1:
             raise ValueError(f"{name} must be 1-D")
@@ -79,7 +98,7 @@ def cg(Ap, Aj, Ax, b, x=None, *, rtol=1e-6, max_iter=None, kind="auto", jacobi=F
     a.stream = (stream if stream is not None else torch.cuda.current_stream(Ap.device)).cuda_stream
     out = _lib.CgOut()
     with torch.cuda.device(Ap.device):
-        st = _lib.lib().spmvb200_cg(C.byref(a), C.byref(out))
-    _lib.check(st, f"spmvb200_cg[{kind}]")
+        st = getattr(_lib.lib(), entry)(C.byref(a), C.byref(out))
+    _lib.check(st, f"{entry}[{kind}]")
     return CgResult(x=x, iterations=int(out.iterations), residual_norm=float(out.residual_norm),
                     b_norm=float(out.b_norm), converged=bool(out.converged), breakdown=bool(out.breakdown))
