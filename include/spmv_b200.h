@@ -244,6 +244,32 @@ SPMVB200_API int spmvb200_cg(const spmvb200_cg_args_t *args, spmvb200_cg_result_
  * spmvb200_release_cache. */
 SPMVB200_API int spmvb200_bicgstab(const spmvb200_cg_args_t *args, spmvb200_cg_result_t *out);
 
+/* ---- restarted GMRES(m) solve A x = b on the device (csrc/gmres.cu) ------------------------
+ * A is n x n in CSR and need not be symmetric; right-preconditioned GMRES(m) with M = I, or
+ * M = diag(A) with SPMVB200_CG_JACOBI: it solves A M^-1 u = b, x = x0 + M^-1 V y, so the residual
+ * it minimises over each Krylov space is the true residual b - A x and rtol means what it means
+ * for spmvb200_cg.  (scipy.sparse.linalg.gmres preconditions on the left.)  Takes the records of
+ * spmvb200_cg with the same meaning, the same argument checks and status codes, and
+ * SPMVB200_ERR_INVALID for `restart` outside [1, SPMVB200_GMRES_MAX_RESTART], checked before any
+ * CUDA call; the cycle length used is m = min(restart, n).  n == 0 reports convergence after 0
+ * iterations.  An Arnoldi step is one SpMV of `kind` (SPMVB200_FLAG_STATIC_PATTERN on every call
+ * after the first) and four streaming kernels, whatever the step's place in the cycle: classical
+ * Gram-Schmidt with one re-orthogonalisation (CGS2), dot products in double in a fixed order, the
+ * Hessenberg matrix and its Givens rotations (r = hypot(a, b)) in double on the device.  A cycle
+ * ends after m steps, when the residual estimate |g_{j+1}| <= rtol * ||b||, at a lucky breakdown
+ * (||w|| after the orthogonalisation <= eps * ||w|| before it, eps of the value type), or at
+ * max_iter; then x += M^-1 V y, and the explicit ||b - A x|| decides convergence, or the next
+ * cycle starts from that residual.  A breakdown (not an error) is a non-finite h, norm or
+ * rotation (x is left at the start of that cycle), a non-finite ||b|| or ||r0|| (NaN or inf in
+ * the input), or a lucky breakdown whose explicit residual still misses the tolerance.
+ * `iterations` counts Arnoldi steps (the SpMVs inside cycles).  The host reads the device flags
+ * once per batch of 1, 2, 4, ... 64 steps; a cycle that ends early on the device leaves the rest
+ * of its m steps idle, and those count against max_iter.  residual_norm is ||b - A x|| of the
+ * returned x, computed once more in fp64.  Workspace ((m + 1) vectors, m + 3 with Jacobi) is
+ * cached per (device, stream) and freed by spmvb200_release_cache. */
+#define SPMVB200_GMRES_MAX_RESTART 64
+SPMVB200_API int spmvb200_gmres(const spmvb200_cg_args_t *args, int32_t restart, spmvb200_cg_result_t *out);
+
 /* ---- merge-path partition, exposed so parity tests can demand bit-exact coordinates --- */
 /* Row coordinate of the merge path on each diagonal min(t * tile_items, n_rows + nnz),
  * t = 0 .. n_coords-1, written to the DEVICE array coords_x (int32).  The nonzero

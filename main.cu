@@ -25,12 +25,15 @@
 //   not converge
 //   --bicgstab RTOL [--jacobi]: the same with one BiCGSTAB solve per kind (spmvb200_bicgstab), for a
 //   square matrix that need not be symmetric
+//   --gmres RTOL [--restart M] [--jacobi]: the same with one restarted GMRES(M) solve per kind
+//   (spmvb200_gmres, M = 20 by default, at most 64), for a square matrix that need not be symmetric
 #include <algorithm>
 #include <chrono>
 #include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <filesystem>
+#include <functional>
 #include <iostream>
 #include <numeric>
 #include <string>
@@ -62,7 +65,9 @@ struct Options {
     int power = 0;   // --power K: K power-iteration steps x <- A x / ||A x|| (BASELINE.json configs[4])
     double cg_rtol = 0;      // --cg RTOL: one CG solve of A x = A*1 per kind
     double bicgstab_rtol = 0;  // --bicgstab RTOL: one BiCGSTAB solve of A x = A*1 per kind
-    bool cg_jacobi = false;  // --jacobi: with M = diag(A) (both solvers)
+    double gmres_rtol = 0;     // --gmres RTOL: one GMRES solve of A x = A*1 per kind
+    int gmres_restart = 20;    // --restart M: GMRES cycle length
+    bool cg_jacobi = false;  // --jacobi: with M = diag(A) (every solver)
 };
 
 template <typename T>
@@ -83,12 +88,12 @@ static int kind_id(const string &k) {
     return -1;
 }
 
-using KrylovSolve = int (*)(const spmvb200_cg_args_t *, spmvb200_cg_result_t *);
+using KrylovSolve = std::function<int(const spmvb200_cg_args_t *, spmvb200_cg_result_t *)>;
 
-// --cg / --bicgstab: b = A*1, x0 = 0, one solve per kind by `solve` (spmvb200_cg or
-// spmvb200_bicgstab); returns the number of kinds that did not converge
+// --cg / --bicgstab / --gmres: b = A*1, x0 = 0, one solve per kind by `solve` (spmvb200_cg,
+// spmvb200_bicgstab or spmvb200_gmres); returns the number of kinds that did not converge
 template <typename offset_t, typename value_t>
-static int run_krylov(const Options &opt, KrylovSolve solve, const char *title, double rtol, index_t n, offset_t nnz,
+static int run_krylov(const Options &opt, const KrylovSolve &solve, const char *title, double rtol, index_t n, offset_t nnz,
                       offset_t *dAp, index_t *dAj, value_t *dAx) {
     const size_t vb = sizeof(value_t);
     vector<value_t> ones((size_t)n, value_t(1)), hx((size_t)n);
@@ -302,7 +307,13 @@ static int run(const Options &opt, const string &name, index_t n_rows, index_t n
         double rtol;
         KrylovSolve solve;
         const char *title;
-    } solves[] = {{opt.cg_rtol, spmvb200_cg, "Conjugate gradients"}, {opt.bicgstab_rtol, spmvb200_bicgstab, "BiCGSTAB"}};
+    } solves[] = {{opt.cg_rtol, spmvb200_cg, "Conjugate gradients"},
+                  {opt.bicgstab_rtol, spmvb200_bicgstab, "BiCGSTAB"},
+                  {opt.gmres_rtol,
+                   [&opt](const spmvb200_cg_args_t *a, spmvb200_cg_result_t *r) {
+                       return spmvb200_gmres(a, opt.gmres_restart, r);
+                   },
+                   "GMRES"}};
     for (const auto &sv : solves) {
         if (sv.rtol <= 0) continue;
         if (n_rows == n_cols) {
@@ -404,7 +415,7 @@ static int run_synthetic(const Options &opt, const string &cfg, long size) {
 int main(int argc, char **argv) {
     if (argc < 3) {
         cerr << "usage: ./bin/<program-name>  <filename.mtx | synthetic:c1..c5[:size]>  <SpMV_kind_string>..."
-                "  [--iters N] [--x ones|random] [--flush] [--dynamic-pattern] [--peak GB/s] [--power K [--gpus N]] [--cg RTOL] [--bicgstab RTOL] [--jacobi]"
+                "  [--iters N] [--x ones|random] [--flush] [--dynamic-pattern] [--peak GB/s] [--power K [--gpus N]] [--cg RTOL] [--bicgstab RTOL] [--gmres RTOL [--restart M]] [--jacobi]"
              << endl;
         exit(1);
     }
@@ -421,6 +432,8 @@ int main(int argc, char **argv) {
         else if (a == "--power" && i + 1 < argc) opt.power = atoi(argv[++i]);
         else if (a == "--cg" && i + 1 < argc) opt.cg_rtol = atof(argv[++i]);
         else if (a == "--bicgstab" && i + 1 < argc) opt.bicgstab_rtol = atof(argv[++i]);
+        else if (a == "--gmres" && i + 1 < argc) opt.gmres_rtol = atof(argv[++i]);
+        else if (a == "--restart" && i + 1 < argc) opt.gmres_restart = atoi(argv[++i]);
         else if (a == "--jacobi") opt.cg_jacobi = true;
         else opt.kinds.push_back(a);
     }

@@ -9,7 +9,8 @@ Python package is the thin binding used by tests, bench.py and the multi-GPU dri
     generate  device-side synthetic matrices (BASELINE.json configs c1..c5)
     matrix    CsrMatrix: host-buffer (end-to-end) front end
     solve     cg(): conjugate-gradient solve on the device (SPD matrices), bicgstab(): BiCGSTAB
-              for general square matrices; both optionally Jacobi-preconditioned
+              and gmres(): restarted GMRES for general square matrices; all optionally
+              Jacobi-preconditioned
 
 Importing the package does not need a GPU; calling into it does, and nothing falls back.
 """

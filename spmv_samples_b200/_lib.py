@@ -18,6 +18,7 @@ OK = 0
 KIND_MERGE, KIND_VECTOR, KIND_LIGHT, KIND_AUTO, KIND_CUSPARSE, KIND_STREAM = 0, 1, 2, 3, 4, 5
 FLAG_STATIC_PATTERN = 1   # SPMVB200_FLAG_STATIC_PATTERN
 CG_JACOBI = 1             # SPMVB200_CG_JACOBI
+GMRES_MAX_RESTART = 64    # SPMVB200_GMRES_MAX_RESTART
 SEMIRINGS = {"plus_times": 0, "min_plus": 1, "max_plus": 2, "or_and": 3}
 MAX_PEERS = 8
 IPC_HANDLE_BYTES = 64
@@ -107,6 +108,8 @@ def lib() -> C.CDLL:
     L.spmvb200_cg.restype = C.c_int
     L.spmvb200_bicgstab.argtypes = [C.POINTER(CgArgs), C.POINTER(CgOut)]
     L.spmvb200_bicgstab.restype = C.c_int
+    L.spmvb200_gmres.argtypes = [C.POINTER(CgArgs), C.c_int32, C.POINTER(CgOut)]
+    L.spmvb200_gmres.restype = C.c_int
     L.spmvb200_launch_count.restype = C.c_int64
     L.spmvb200_get_option.restype = C.c_int64
     L.spmvb200_get_option.argtypes = [C.c_char_p]

@@ -165,12 +165,12 @@ int spmvb200_spmm(const spmvb200_spmm_args_t *a) {
     return SPMVB200_ERR_UNSUPPORTED;
 }
 
-// ---- Krylov solvers: conjugate gradients, BiCGSTAB -----------------------------------------
-// Every argument is checked here, before any CUDA call (so also without a device); then the
-// solver for the offset and value widths runs.
-using KrylovSolve = int (*)(const spmvb200_cg_args_t &, spmvb200_cg_result_t *);
-static int krylov_entry(const spmvb200_cg_args_t *a, spmvb200_cg_result_t *out, KrylovSolve o32_f32,
-                        KrylovSolve o32_f64, KrylovSolve o64_f32, KrylovSolve o64_f64) {
+// ---- Krylov solvers: conjugate gradients, BiCGSTAB, GMRES -----------------------------------
+// Every argument is checked here, before any CUDA call (so also without a device); then
+// solve(OffT(), ValT()) runs the solver for the offset and value widths.
+extern "C++" {
+template <typename Solve>
+static int krylov_entry(const spmvb200_cg_args_t *a, spmvb200_cg_result_t *out, Solve solve) {
     if (!a || !out) return SPMVB200_ERR_INVALID;
     if (a->kind < SPMVB200_KIND_MERGE || a->kind > SPMVB200_KIND_STREAM) return SPMVB200_ERR_INVALID;
     if (a->flags & ~SPMVB200_CG_JACOBI) return SPMVB200_ERR_INVALID;
@@ -187,18 +187,23 @@ static int krylov_entry(const spmvb200_cg_args_t *a, spmvb200_cg_result_t *out, 
     if (!a->Ap || !a->b || !a->x || (a->nnz > 0 && (!a->Aj || !a->Ax))) return SPMVB200_ERR_INVALID;
     if (a->x == a->b) return SPMVB200_ERR_INVALID;
     if (!aligned16(a->Ap) || !aligned16(a->Aj) || !aligned16(a->Ax)) return SPMVB200_ERR_ALIGNMENT;
-    if (a->offset_bits == 32) return a->value_bits == 32 ? o32_f32(*a, out) : o32_f64(*a, out);
-    return a->value_bits == 32 ? o64_f32(*a, out) : o64_f64(*a, out);
+    if (a->offset_bits == 32) return a->value_bits == 32 ? solve(int32_t(), float()) : solve(int32_t(), double());
+    return a->value_bits == 32 ? solve(int64_t(), float()) : solve(int64_t(), double());
+}
 }
 
 int spmvb200_cg(const spmvb200_cg_args_t *a, spmvb200_cg_result_t *out) {
-    return krylov_entry(a, out, cg_solve<int32_t, float>, cg_solve<int32_t, double>, cg_solve<int64_t, float>,
-                        cg_solve<int64_t, double>);
+    return krylov_entry(a, out, [&](auto o, auto v) { return cg_solve<decltype(o), decltype(v)>(*a, out); });
 }
 
 int spmvb200_bicgstab(const spmvb200_cg_args_t *a, spmvb200_cg_result_t *out) {
-    return krylov_entry(a, out, bicgstab_solve<int32_t, float>, bicgstab_solve<int32_t, double>,
-                        bicgstab_solve<int64_t, float>, bicgstab_solve<int64_t, double>);
+    return krylov_entry(a, out, [&](auto o, auto v) { return bicgstab_solve<decltype(o), decltype(v)>(*a, out); });
+}
+
+int spmvb200_gmres(const spmvb200_cg_args_t *a, int32_t restart, spmvb200_cg_result_t *out) {
+    if (restart < 1 || restart > SPMVB200_GMRES_MAX_RESTART) return SPMVB200_ERR_INVALID;
+    return krylov_entry(a, out,
+                        [&](auto o, auto v) { return gmres_solve<decltype(o), decltype(v)>(*a, restart, out); });
 }
 
 // ---- partition / row split -----------------------------------------------------------------

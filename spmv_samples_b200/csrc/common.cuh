@@ -60,7 +60,8 @@ int apply_carveout(const void *kernel, int64_t percent);
 // Slots keep independent buffers so a kernel can hold several at once.
 enum ScratchSlot { SCRATCH_COORDS = 0, SCRATCH_CARRY_ROW, SCRATCH_CARRY_VAL, SCRATCH_COUNTER,
                    SCRATCH_STATS, SCRATCH_MISC, SCRATCH_SPMM_X, SCRATCH_SPMM_Y, SCRATCH_XHOT, SCRATCH_NORM,
-                   SCRATCH_CG, SCRATCH_ROW_END, SCRATCH_START_MASK, SCRATCH_BICGSTAB, SCRATCH_NUM_SLOTS };
+                   SCRATCH_CG, SCRATCH_ROW_END, SCRATCH_START_MASK, SCRATCH_BICGSTAB, SCRATCH_GMRES,
+                   SCRATCH_NUM_SLOTS };
 int scratch_get(cudaStream_t stream, ScratchSlot slot, size_t bytes, void **out);
 
 // What the last merge-path partition launched on a (device, stream) wrote, and where: lets a
@@ -160,6 +161,9 @@ int cg_solve(const spmvb200_cg_args_t &a, spmvb200_cg_result_t *out);
 // BiCGSTAB (bicgstab.cu); arguments checked by the caller
 template <typename OffT, typename ValT>
 int bicgstab_solve(const spmvb200_cg_args_t &a, spmvb200_cg_result_t *out);
+// restarted GMRES (gmres.cu); arguments, restart included, checked by the caller
+template <typename OffT, typename ValT>
+int gmres_solve(const spmvb200_cg_args_t &a, int restart, spmvb200_cg_result_t *out);
 
 // The hot part of x, compacted (hotx.cu): a per-matrix plan holding a remapped copy of Aj (hot
 // column c stored as 0x80000000 | rank) and the list of hot columns; x_hot lives in the

@@ -1,6 +1,6 @@
-// krylov.cuh -- pieces the device-resident Krylov solvers (cg.cu, bicgstab.cu) share: the
-// fixed-order fp64 block and grid reductions, the Jacobi diagonal, the fp64 true residual, the
-// SpMV call on the solver's arguments and the read of a solver's device state block.
+// krylov.cuh -- pieces the device-resident Krylov solvers (cg.cu, bicgstab.cu, gmres.cu) share:
+// the fixed-order fp64 block and grid reductions, the Jacobi diagonal, the fp64 true residual,
+// the SpMV call on the solver's arguments and the read of a solver's device state block.
 //
 // Every dot product accumulates in double in a fixed order: per-block partials, then the last
 // block to finish (threadfence + counter, as norm_exchange_kernel in power.cu) adds them in block
@@ -62,6 +62,56 @@ __device__ __forceinline__ bool grid_sum(double (&v)[N], double *partial, unsign
         for (int i = threadIdx.x; i < (int)gridDim.x; i += kKrylovBlock) v[j] += __ldcg(partial + (size_t)j * gridDim.x + i);
     }
     block_sum<N>(v);
+    if (threadIdx.x == 0) *counter = 0;  // ready for the next reduction
+    return true;
+}
+
+// Sums whose count is known only at run time (GMRES: one dot product per basis vector).  Each
+// warp adds its lanes' terms in the shuffle order of block_sum and keeps a running total per sum
+// in shared memory, s[c * kKrylovWarps + warp]; grid_sum_n then adds the warps in order, writes
+// one partial per block and sum, and the last block to finish adds the partials in block order,
+// as grid_sum does.  Every thread of the block calls both, with warp-uniform control flow.
+constexpr int kKrylovWarps = kKrylovBlock / 32;
+
+__device__ __forceinline__ void warp_accumulate(double v, double *s_c) {
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
+    if ((threadIdx.x & 31) == 0) s_c[threadIdx.x >> 5] += v;
+}
+
+// The `count` totals of the running warp sums in s: true in the last block to finish, where
+// tot[0 .. count) (shared) then holds them for every thread.  s is overwritten.
+__device__ __forceinline__ bool grid_sum_n(int count, double *s, double *tot, double *partial,
+                                           unsigned int *counter) {
+    __shared__ bool is_last;
+    __syncthreads();
+    for (int c = threadIdx.x; c < count; c += kKrylovBlock) {
+        double t = 0.0;
+#pragma unroll
+        for (int w = 0; w < kKrylovWarps; ++w) t += s[c * kKrylovWarps + w];
+        partial[(size_t)c * gridDim.x + blockIdx.x] = t;
+    }
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) is_last = atomicAdd(counter, 1u) == gridDim.x - 1;
+    __syncthreads();
+    if (!is_last) return false;
+    __threadfence();
+    for (int c = 0; c < count; ++c) {
+        double v = 0.0;
+        for (int i = threadIdx.x; i < (int)gridDim.x; i += kKrylovBlock) v += __ldcg(partial + (size_t)c * gridDim.x + i);
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
+        if ((threadIdx.x & 31) == 0) s[c * kKrylovWarps + (threadIdx.x >> 5)] = v;
+    }
+    __syncthreads();
+    for (int c = threadIdx.x; c < count; c += kKrylovBlock) {
+        double t = 0.0;
+#pragma unroll
+        for (int w = 0; w < kKrylovWarps; ++w) t += s[c * kKrylovWarps + w];
+        tot[c] = t;
+    }
+    __syncthreads();
     if (threadIdx.x == 0) *counter = 0;  // ready for the next reduction
     return true;
 }

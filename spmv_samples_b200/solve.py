@@ -1,17 +1,20 @@
 """Krylov solves of A x = b on the device: conjugate gradients (spmvb200_cg, csrc/cg.cu) for a
-symmetric positive definite A, BiCGSTAB (spmvb200_bicgstab, csrc/bicgstab.cu) for any square A.
+symmetric positive definite A; BiCGSTAB (spmvb200_bicgstab, csrc/bicgstab.cu) and restarted
+GMRES (spmvb200_gmres, csrc/gmres.cu) for any square A.
 
     res = cg(Ap, Aj, Ax, b, rtol=1e-8, kind="auto", jacobi=True)
     res = bicgstab(Ap, Aj, Ax, b, rtol=1e-8, kind="auto", jacobi=True)
+    res = gmres(Ap, Aj, Ax, b, rtol=1e-8, restart=30, kind="auto", jacobi=True)
 
 A is an n x n CSR matrix (CUDA tensors, as for spmv.SpMV).  A CG iteration is one SpMV of the
-chosen kind and three streaming kernels, a BiCGSTAB iteration two SpMVs and five; the dot
-products accumulate in double in a fixed order, and the host reads the convergence flags once
+chosen kind and three streaming kernels, a BiCGSTAB iteration two SpMVs and five, a GMRES step
+one SpMV and four; the dot products accumulate in double in a fixed order, and the host reads the convergence flags once
 per batch of iterations instead of once per iteration.  There is no PyTorch or CPU fallback.
 """
 from __future__ import annotations
 
 import ctypes as C
+import numbers
 from dataclasses import dataclass
 
 import torch
@@ -26,8 +29,8 @@ class CgResult:
     iterations: int
     residual_norm: float   # ||b - A x|| of the returned x, computed in fp64
     b_norm: float
-    converged: bool        # ||r|| <= rtol * ||b|| for the recursive residual r
-    breakdown: bool        # the method cannot continue (not an error): see cg() and bicgstab()
+    converged: bool        # ||r|| <= rtol * ||b||: the recursive r (cg, bicgstab), the explicit one (gmres)
+    breakdown: bool        # the method cannot continue (not an error): see each solver
 
 
 def cg(Ap, Aj, Ax, b, x=None, *, rtol=1e-6, max_iter=None, kind="auto", jacobi=False,
@@ -52,8 +55,28 @@ def bicgstab(Ap, Aj, Ax, b, x=None, *, rtol=1e-6, max_iter=None, kind="auto", ja
     return _solve("spmvb200_bicgstab", Ap, Aj, Ax, b, x, rtol, max_iter, kind, jacobi, stream)
 
 
-def _solve(entry, Ap, Aj, Ax, b, x, rtol, max_iter, kind, jacobi, stream) -> CgResult:
-    """Both solvers: the argument checks, made before touching a device, then the call."""
+def gmres(Ap, Aj, Ax, b, x=None, *, rtol=1e-6, restart=20, max_iter=None, kind="auto", jacobi=False,
+          stream=None) -> CgResult:
+    """Solve A x = b for a general square A by right-preconditioned restarted GMRES(restart), with
+    M = diag(A) when jacobi=True.  Right preconditioning minimises the true residual, so rtol
+    means what it means for cg() (scipy.sparse.linalg.gmres preconditions on the left).  Each
+    cycle orthogonalises by classical Gram-Schmidt with one re-orthogonalisation and ends after
+    min(restart, n) steps, when the residual estimate meets rtol * ||b||, or at a lucky breakdown;
+    then the explicit ||b - A x|| decides convergence or starts the next cycle.  restart: 1 to 64.
+    x: initial guess, overwritten with the solution; None starts from zero.  max_iter: the cap on
+    Arnoldi steps, which `iterations` counts (the idle rest of a cycle that ended early counts
+    against it); None means n.  A breakdown is a non-finite value in the method (x is left at the
+    start of that cycle) or a lucky breakdown whose explicit residual misses the tolerance.
+    Raises ValueError for a restart outside [1, 64], and SpmvB200Error (status 1) when
+    jacobi=True and a diagonal entry is missing or zero."""
+    if isinstance(restart, bool) or not isinstance(restart, numbers.Integral) or not 1 <= restart <= _lib.GMRES_MAX_RESTART:
+        raise ValueError(f"restart must be an integer in [1, {_lib.GMRES_MAX_RESTART}]")
+    return _solve("spmvb200_gmres", Ap, Aj, Ax, b, x, rtol, max_iter, kind, jacobi, stream, int(restart))
+
+
+def _solve(entry, Ap, Aj, Ax, b, x, rtol, max_iter, kind, jacobi, stream, *extra) -> CgResult:
+    """Every solver: the argument checks, made before touching a device, then the call, with the
+    solver's own arguments (`extra`) between the records."""
     for name, t in (("Ap", Ap), ("Aj", Aj), ("Ax", Ax), ("b", b), ("x", x)):
         if t is not None and t.dim() != 1:
             raise ValueError(f"{name} must be 1-D")
@@ -98,7 +121,7 @@ def _solve(entry, Ap, Aj, Ax, b, x, rtol, max_iter, kind, jacobi, stream) -> CgR
     a.stream = (stream if stream is not None else torch.cuda.current_stream(Ap.device)).cuda_stream
     out = _lib.CgOut()
     with torch.cuda.device(Ap.device):
-        st = getattr(_lib.lib(), entry)(C.byref(a), C.byref(out))
+        st = getattr(_lib.lib(), entry)(C.byref(a), *extra, C.byref(out))
     _lib.check(st, f"{entry}[{kind}]")
     return CgResult(x=x, iterations=int(out.iterations), residual_norm=float(out.residual_norm),
                     b_norm=float(out.b_norm), converged=bool(out.converged), breakdown=bool(out.breakdown))
