@@ -62,13 +62,13 @@ def jacobi_dinv(Ap, Aj, Ax):
     return 1.0 / np.bincount(rows[on], weights=Ax[on].astype(np.float64), minlength=n)
 
 
-def bicgstab_reference(Ap, Aj, Ax, b, rtol, max_iter, dinv=None, x0=None):
+def bicgstab_reference(Ap, Aj, Ax, b, rtol, max_iter, dinv=None, x0=None, trace=None):
     """Right-preconditioned BiCGSTAB in fp64 on oracle.cpu.spmv_fp64, in the operation order of
     scipy.sparse.linalg.bicgstab, with the stopping rules of csrc/bicgstab.cu: converged when
     ||r|| <= rtol * ||b|| at the start or after an iteration, or ||s|| <= rtol * ||b|| at the
     half step (which counts as an iteration); breakdown at an exact zero or a non-finite value of
-    rho, (r^, v), alpha, (t, t) or omega, or at omega == 0.  Returns (x, iterations, converged,
-    breakdown)."""
+    rho, (r^, v), alpha, (t, t) or omega, or at omega == 0.  trace, a list, gets every ||r|| and
+    ||s|| compared with the tolerance.  Returns (x, iterations, converged, breakdown)."""
     n = Ap.shape[0] - 1
     b = np.asarray(b, dtype=np.float64)
     x = np.zeros(n) if x0 is None else np.array(x0, dtype=np.float64)
@@ -79,6 +79,11 @@ def bicgstab_reference(Ap, Aj, Ax, b, rtol, max_iter, dinv=None, x0=None):
     def M(v):
         return v if dinv is None else dinv * v
 
+    def decides(v):
+        if trace is not None:
+            trace.append(np.linalg.norm(v))
+        return np.linalg.norm(v) <= tol
+
     with np.errstate(all="ignore"):
         r = b - A(x)
         rh = r.copy()
@@ -86,7 +91,7 @@ def bicgstab_reference(Ap, Aj, Ax, b, rtol, max_iter, dinv=None, x0=None):
         tol = rtol * bnorm
         if bnorm == 0:
             return np.zeros(n), 0, True, False
-        if np.linalg.norm(r) <= tol:
+        if decides(r):
             return x, 0, True, False
         rho = rh @ r
         if rho == 0 or not np.isfinite(rho):
@@ -103,7 +108,7 @@ def bicgstab_reference(Ap, Aj, Ax, b, rtol, max_iter, dinv=None, x0=None):
             s = r - alpha * v
             x = x + alpha * ph
             it += 1
-            if np.linalg.norm(s) <= tol:
+            if decides(s):
                 return x, it, True, False
             sh = M(s)
             t = A(sh)
@@ -113,7 +118,7 @@ def bicgstab_reference(Ap, Aj, Ax, b, rtol, max_iter, dinv=None, x0=None):
                 return x, it, False, True
             x = x + omega * sh
             r = s - omega * t
-            if np.linalg.norm(r) <= tol:
+            if decides(r):
                 return x, it, True, False
             rho_new = rh @ r
             if omega == 0 or rho_new == 0 or not np.isfinite(rho_new):

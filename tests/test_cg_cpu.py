@@ -11,10 +11,11 @@ from oracle import cpu
 from oracle import generators as g
 
 
-def pcg_reference(Ap, Aj, Ax, b, rtol, max_iter, dinv=None, x0=None):
+def pcg_reference(Ap, Aj, Ax, b, rtol, max_iter, dinv=None, x0=None, trace=None):
     """Preconditioned CG (Hestenes-Stiefel) in fp64 on oracle.cpu.spmv_fp64, with the stopping
     rules of csrc/cg.cu: converged when ||r|| <= rtol * ||b|| after an update (or at the start),
-    breakdown when p.q <= 0.  Returns (x, iterations, converged, breakdown)."""
+    breakdown when p.q <= 0.  trace, a list, gets every ||r|| compared with the tolerance.
+    Returns (x, iterations, converged, breakdown)."""
     n = Ap.shape[0] - 1
     b = np.asarray(b, dtype=np.float64)
     x = np.zeros(n) if x0 is None else np.array(x0, dtype=np.float64)
@@ -25,6 +26,8 @@ def pcg_reference(Ap, Aj, Ax, b, rtol, max_iter, dinv=None, x0=None):
     tol = rtol * np.linalg.norm(b)
     if np.linalg.norm(b) == 0:
         return np.zeros(n), 0, True, False
+    if trace is not None:
+        trace.append(np.linalg.norm(r))
     if np.linalg.norm(r) <= tol:
         return x, 0, True, False
     it = 0
@@ -37,6 +40,8 @@ def pcg_reference(Ap, Aj, Ax, b, rtol, max_iter, dinv=None, x0=None):
         x = x + alpha * p
         r = r - alpha * q
         it += 1
+        if trace is not None:
+            trace.append(np.linalg.norm(r))
         if np.linalg.norm(r) <= tol:
             return x, it, True, False
         z = r if dinv is None else dinv * r
